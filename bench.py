@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W             # our arm (CUDA kernels)
     python bench.py --impl reference --steps K --warmup W     # reference arm: CPU oracle port
+    python bench.py --steps K --warmup W --dump-outputs DIR   # + what the last timed epoch computed, as DIR/<name>.npy
 
 Metric (BASELINE.json): **KGAT epoch seconds** -- one "step" is one reference epoch body
 (main.py:290-361: n_cf CF steps + n_kg KG steps + one attention refresh) over pre-sampled synthetic
@@ -106,6 +107,8 @@ def reference_model(g, params, device):
 
     mods = build_ref.load()
     if mods is None:
+        print("bench.py: oracle/_ref is not staged (build() with KGAT_REFERENCE set stages it): the baselines run the oracle port",
+              file=sys.stderr)
         return None
     ref, _ = mods
     m = ref.KGAT(ref.KGATArgs(user_num=g.user_num, entity_num=g.entity_num, relation_num=g.relation_num, attentive_matrix=_att_coo(g)))
@@ -459,6 +462,30 @@ def c5_scaled_block(dev, peak):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_ATT_ENTRIES = 1 << 20
+
+
+def dump_outputs(out_dir: Path, model, losses) -> None:
+    """What ``TrainEngine.run_epoch`` leaves its caller after the last timed epoch: the epoch's mean CF and KG losses and the
+    trained model -- every dense parameter in full, and the refreshed attention weights at a fixed, seeded sample of their
+    entries (all of them would not fit the dump's 64 MB next to the entity table).  The inputs and the gradients' summation
+    order are fixed, so two runs of one build with the same arguments write bit-identical arrays."""
+    arrays = {"cf_loss": np.array(losses[0], np.float64), "kg_loss": np.array(losses[1], np.float64)}
+    for k, v in model.state_dict().items():
+        if not v.is_sparse:
+            arrays[k] = v.detach().float().cpu().numpy()
+    vals = model.attentive_matrix.data._values()
+    pick = np.sort(np.random.default_rng(0).choice(vals.numel(), size=min(DUMP_ATT_ENTRIES, vals.numel()), replace=False))
+    arrays["attentive_matrix.values_sample"] = vals[torch.from_numpy(pick).to(vals.device)].float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out_dir / f"{k}.npy", a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -470,7 +497,13 @@ def main():
     ap.add_argument("--no-hbm-regime", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary shapes (Yelp2018 top-20, scaled C5, full Codeforces)")
     ap.add_argument("--budget-s", type=float, default=330.0, help="wall-clock budget: optional blocks are skipped once it is spent")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write what the last timed epoch left the caller (losses, trained parameters, refreshed attention) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs covers the single-GPU run of our implementation")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -533,6 +566,8 @@ def main():
         t1.record()
         barrier()
     launches = _lib.LaunchCounter.count
+    if args.dump_outputs is not None:  # before the e2e leg below trains the same model further
+        dump_outputs(args.dump_outputs, model, losses)
     phases = dict(engine.last_phase_ms)
     epoch_s = t0.elapsed_time(t1) / 1e3 / max(args.steps, 1)
     clk = clocks.summary()

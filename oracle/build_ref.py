@@ -1,14 +1,13 @@
 """Recipe for ``oracle/_ref``: the UNMODIFIED reference modules of the hot path, staged for the GPU box.
 
-    python oracle/build_ref.py            # build container only; a no-op with a notice when /root/reference is absent
+    python oracle/build_ref.py <checkout of the reference repository>
 
 The reference is pure Python (no compile step), so "building" it means staging, byte for byte, the
 handful of modules the KGAT hot path consists of -- ``src/model/KGAT/{model, aggregator,
 multi_head_attention, preprocess}.py``, ``src/utils/metrics_calculator.py`` and the small modules
 they import (``src/type.py``, ``src/constants.py``, ``src/utils/{kg_triplets_generator,
-json_writer}.py``) plus the package ``__init__`` files -- from where they lie under
-``/root/reference`` into ``oracle/_ref/`` (git-ignored, NOT gpurun-ignored: it travels to the GPU box
-like a built ``.so``).  Nothing is edited; ``MANIFEST.json`` records the sha256 of every staged file
+json_writer}.py``) plus the package ``__init__`` files -- from where they lie in a checkout of the
+reference into ``oracle/_ref/`` (git-ignored).  Nothing is edited; ``MANIFEST.json`` records the sha256 of every staged file
 so the bench line can say exactly which bytes were timed.
 
 Users: ``bench.py --impl reference`` / the ``cpu_baseline`` and ``gpu_incumbent`` legs (the reference's
@@ -24,7 +23,6 @@ import shutil
 import sys
 from pathlib import Path
 
-REF = Path("/root/reference")
 OUT = Path(__file__).resolve().parent / "_ref"
 
 FILES = [
@@ -44,14 +42,10 @@ FILES = [
 ]
 
 
-def build(quiet: bool = False) -> bool:
-    if not REF.is_dir():
-        if not quiet:
-            print(f"oracle/build_ref.py: {REF} not present (GPU box?) -- keeping the staged oracle/_ref as is")
-        return OUT.is_dir()
+def build(ref: Path, quiet: bool = False) -> bool:
     manifest = {}
     for rel in FILES:
-        src, dst = REF / rel, OUT / rel
+        src, dst = ref / rel, OUT / rel
         if not src.exists():
             if rel.endswith("__init__.py"):  # namespace-style package in the reference: an empty marker is equivalent
                 dst.parent.mkdir(parents=True, exist_ok=True)
@@ -62,7 +56,7 @@ def build(quiet: bool = False) -> bool:
         dst.parent.mkdir(parents=True, exist_ok=True)
         shutil.copyfile(src, dst)
         manifest[rel] = hashlib.sha256(dst.read_bytes()).hexdigest()
-    (OUT / "MANIFEST.json").write_text(json.dumps({"source": str(REF), "files": manifest}, indent=1) + "\n")
+    (OUT / "MANIFEST.json").write_text(json.dumps({"source": str(ref), "files": manifest}, indent=1) + "\n")
     if not quiet:
         print(f"oracle/_ref: staged {len(manifest)} unmodified reference files")
     return True
@@ -88,4 +82,6 @@ def load():
 
 
 if __name__ == "__main__":
-    build()
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: python oracle/build_ref.py <checkout of the reference repository>")
+    build(Path(sys.argv[1]).resolve())

@@ -1,12 +1,10 @@
 """Generate the golden vectors under tests/golden/ by running the UNMODIFIED reference.
 
-Run in the build container only (``/root/reference`` does not exist on the GPU box):
-
-    python oracle/make_golden.py
+    python oracle/make_golden.py <checkout of the reference repository>
 
 It imports ``src.model.KGAT.{model,preprocess}`` and ``src.utils.metrics_calculator`` from
-``/root/reference`` (read-only; bytecode writing disabled), drives them with seeded inputs and
-stores inputs + outputs as ``.npz`` files.  The reference publishes no golden vectors of its own
+that checkout (read-only; bytecode writing disabled), drives them with seeded inputs and
+stores inputs + outputs as ``.npz`` files (``oracle/golden_io.py``: files above 1 MB are stored compacted).  The reference publishes no golden vectors of its own
 (SURVEY.md section 8c), so these files are what pins the oracle and the CUDA path to the reference.
 
 TEST INFRASTRUCTURE - not product code.
@@ -25,7 +23,9 @@ import numpy as np
 
 sys.dont_write_bytecode = True
 REPO = Path(__file__).resolve().parents[1]
-REF = Path("/root/reference")
+if len(sys.argv) != 2:
+    raise SystemExit("usage: python oracle/make_golden.py <checkout of the reference repository>")
+REF = Path(sys.argv[1]).resolve()
 sys.path.insert(0, str(REF))
 sys.path.insert(0, str(REPO))
 
@@ -33,6 +33,7 @@ import torch  # noqa: E402
 import torch.nn.functional as F  # noqa: E402
 
 pkg = importlib.import_module("problem-recommender-system-using-kgat-in-codeforces_b200.synthetic")
+from oracle import golden_io  # noqa: E402
 
 from src.model.KGAT import preprocess as ref_pre  # noqa: E402
 from src.model.KGAT.model import KGAT, KGATArgs, KGATMode  # noqa: E402
@@ -176,7 +177,7 @@ def grads_of(model, names):
     return {"grad::" + n: sd[n].grad.detach().clone().numpy() for n in names if sd[n].grad is not None}
 
 
-def golden_model(tag: str, shape: str, dup: int, cf_b: int, kg_b: int, n_pred_users: int):
+def golden_model(tag: str, shape: str, dup: int, cf_b: int, kg_b: int, n_pred_users: int, sample: dict | None = None):
     g = pkg.make_ckg(shape, seed=SEED, duplicate_pairs=dup)
     n = g.node_num
     torch.manual_seed(SEED)
@@ -317,6 +318,8 @@ def golden_model(tag: str, shape: str, dup: int, cf_b: int, kg_b: int, n_pred_us
     out["traj_losses"] = np.array(losses, np.float64)
     out.update({"traj_" + k: v for k, v in sd_to_np(model.state_dict()).items() if "multi_head" not in k})
     out["traj_att_values"] = model.attentive_matrix.data._values().numpy()
+    if sample:  # keeps the file under 1 MB: inputs as digests + recipe, the largest outputs as a seeded row sample
+        out = golden_io.compact(out, (shape, SEED, dup), sample)
     np.savez_compressed(OUT / f"model_{tag}.npz", **out)
     size = (OUT / f"model_{tag}.npz").stat().st_size
     print(f"model_{tag}: N={n} nnz={g.nnz} att_nnz={g.att_rows.size} R={g.relation_num} file={size / 1e6:.2f} MB losses={losses}")
@@ -382,5 +385,8 @@ if __name__ == "__main__":
     golden_preprocess()
     golden_model("tiny", "tiny", dup=0, cf_b=16, kg_b=32, n_pred_users=8)
     golden_model("tiny_dup", "tiny", dup=40, cf_b=16, kg_b=32, n_pred_users=8)
-    golden_model("small", "small", dup=0, cf_b=64, kg_b=128, n_pred_users=16)
+    E = "_user_entity_embedding.weight"
+    golden_model("small", "small", dup=0, cf_b=64, kg_b=128, n_pred_users=16,
+                 sample={"all_embeddings_eval": 256, **{f"{p}::{E}": 256 for p in ("cf_eval_grad", "cf_train_grad", "kg_grad", "traj_param")},
+                         "kg_grad::_trans_matrix": 6, "traj_param::_trans_matrix": 6})
     golden_training()

@@ -163,8 +163,8 @@ KERNELS_PER_CALL = {
     "kgat_att_edge_weights": 1, "kgat_gather_concat": 1, "kgat_sgemm_nt": 1, "kgat_mask_scores": 1, "kgat_topk_rows": 1,
     "kgat_adam_advance": 1, "kgat_adam_set_hyper": 1, "kgat_adam_apply": 1, "kgat_adam_hyper_table": 1, "kgat_adam_lazy_catchup": 1, "kgat_adam_sparse_rows": 1,
     "kgat_adam_lazy_flush": 1, "kgat_fill_f32": 1, "kgat_select_batch_i64": 1, "kgat_sample_cf_batch": 1, "kgat_sample_kg_batch": 1,
-    "kgat_peer_push": 1, "kgat_peer_push_rows": 1, "kgat_publish_loss": 1, "kgat_zero_rows_i64": 1, "kgat_transr_rows_to_dense": 1, "kgat_transr_release_rows": 1, "kgat_peer_signal_wait": 1, "kgat_transr_claim_rows": 1, "kgat_transr_step": 3,
-    "kgat_adam_rolling_prepare": 1, "kgat_transr_step_claimed": 2, "kgat_adam_rolling_apply": 1, "kgat_selftest_adam_arith": 1, "kgat_step_begin_i64": 1,
+    "kgat_peer_push": 1, "kgat_peer_push_rows": 1, "kgat_publish_loss": 1, "kgat_zero_rows_i64": 1, "kgat_transr_rows_to_dense": 1, "kgat_transr_release_rows": 1, "kgat_peer_signal_wait": 1, "kgat_transr_claim_rows": 1, "kgat_transr_step": 4,
+    "kgat_adam_rolling_prepare": 1, "kgat_transr_step_claimed": 3, "kgat_adam_rolling_apply": 1, "kgat_selftest_adam_arith": 1, "kgat_step_begin_i64": 1,
 }
 
 

@@ -97,38 +97,86 @@ __global__ void __launch_bounds__(256) bpr_fwd_kernel(Tables T, const int64_t* _
     }
 }
 
+__device__ __forceinline__ int64_t slot_id(const int64_t* __restrict__ a, const int64_t* __restrict__ b, const int64_t* __restrict__ c,
+                                           int batch, int e) {
+    return e < batch ? a[e] : (e < 2 * batch ? b[e - batch] : c[e - 2 * batch]);
+}
+
+// Contribution of batch slot k (sample k mod B; role user / positive / negative) to its node's gradient, features [4f, 4f + 4)
+__device__ __forceinline__ void bpr_slot_grad(const float* __restrict__ tab, int64_t ld, const int64_t* __restrict__ users,
+                                              const int64_t* __restrict__ pos, const int64_t* __restrict__ neg, int batch,
+                                              const float* __restrict__ scratch, float g, float lam, int k, int f, float4& acc) {
+    const int b = k % batch, role = k / batch;
+    const float s = sigmoidf_(-scratch[b]) * g;  // d(-logsigmoid(m))/dm = -sigmoid(-m)
+    const float4 a = ldg4(tab + users[b] * ld + f * 4);
+    const float4 x = ldg4(tab + pos[b] * ld + f * 4);
+    const float4 y = ldg4(tab + neg[b] * ld + f * 4);
+    if (role == 0) {
+        acc.x += s * (y.x - x.x) + lam * a.x; acc.y += s * (y.y - x.y) + lam * a.y;
+        acc.z += s * (y.z - x.z) + lam * a.z; acc.w += s * (y.w - x.w) + lam * a.w;
+    } else if (role == 1) {
+        acc.x += -s * a.x + lam * x.x; acc.y += -s * a.y + lam * x.y;
+        acc.z += -s * a.z + lam * x.z; acc.w += -s * a.w + lam * x.w;
+    } else {
+        acc.x += s * a.x + lam * y.x; acc.y += s * a.y + lam * y.y;
+        acc.z += s * a.z + lam * y.z; acc.w += s * a.w + lam * y.w;
+    }
+}
+
+// One warp per id slot e of the batch (users, then positives, then negatives).  The warp of the FIRST slot holding a node
+// sums the contributions of every slot holding it, in slot order, and adds the sum to the node's gradient row: a fixed
+// summation order, so the gradients are bit-identical from run to run (float atomics would add in arrival order).  One pass
+// over the slots decides ownership and lists the node's slots (lane q keeps the q-th); a node held by more than 32 slots
+// rescans them per feature chunk instead.
 __global__ void __launch_bounds__(256) bpr_bwd_kernel(Tables T, GradTables G, const int64_t* __restrict__ users,
                                                       const int64_t* __restrict__ pos, const int64_t* __restrict__ neg, int batch,
                                                       float reg, const float* __restrict__ scratch,
                                                       const float* __restrict__ g_loss) {
     const int lane = threadIdx.x & 31;
-    const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (b >= batch) return;
-    const int64_t u = users[b], p = pos[b], n = neg[b];
+    const int e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int n3 = 3 * batch;
+    if (e >= n3) return;
+    const int64_t id = slot_id(users, pos, neg, batch, e);
+    int my_slot = -1, n_match = 0;
+    for (int k0 = 0; k0 < n3; k0 += 32) {
+        const int k = k0 + lane;
+        const unsigned bal = __ballot_sync(kFull, k < n3 && slot_id(users, pos, neg, batch, k) == id);
+        const unsigned before = e - k0 >= 32 ? kFull : (e > k0 ? (1u << (e - k0)) - 1u : 0u);
+        if (bal & before) return;  // an earlier slot holds the node: its warp owns the row
+        for (unsigned rest = bal; rest; rest &= rest - 1) {
+            const int src = __ffs(rest) - 1;
+            if (n_match + __popc(bal & ((1u << src) - 1u)) == lane) my_slot = k0 + src;
+        }
+        n_match += __popc(bal);
+    }
     const float g = g_loss[0] / (float)batch;
-    const float s = sigmoidf_(-scratch[b]) * g;  // d(-logsigmoid(m))/dm = -sigmoid(-m)
     const float lam = reg * g;
     for (int t = 0; t < T.n; ++t) {
         if (G.p[t] == nullptr) continue;
-        for (int f = lane; f < T.q[t]; f += 32) {
-            const float4 a = ldg4(T.p[t] + u * T.ld[t] + f * 4);
-            const float4 x = ldg4(T.p[t] + p * T.ld[t] + f * 4);
-            const float4 y = ldg4(T.p[t] + n * T.ld[t] + f * 4);
-            float* gu = G.p[t] + u * G.ld[t] + f * 4;
-            float* gp = G.p[t] + p * G.ld[t] + f * 4;
-            float* gn = G.p[t] + n * G.ld[t] + f * 4;
-            atomicAdd(gu + 0, s * (y.x - x.x) + lam * a.x);
-            atomicAdd(gu + 1, s * (y.y - x.y) + lam * a.y);
-            atomicAdd(gu + 2, s * (y.z - x.z) + lam * a.z);
-            atomicAdd(gu + 3, s * (y.w - x.w) + lam * a.w);
-            atomicAdd(gp + 0, -s * a.x + lam * x.x);
-            atomicAdd(gp + 1, -s * a.y + lam * x.y);
-            atomicAdd(gp + 2, -s * a.z + lam * x.z);
-            atomicAdd(gp + 3, -s * a.w + lam * x.w);
-            atomicAdd(gn + 0, s * a.x + lam * y.x);
-            atomicAdd(gn + 1, s * a.y + lam * y.y);
-            atomicAdd(gn + 2, s * a.z + lam * y.z);
-            atomicAdd(gn + 3, s * a.w + lam * y.w);
+        for (int f = lane; f - lane < T.q[t]; f += 32) {
+            float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (n_match <= 32) {
+                for (int q = 0; q < n_match; ++q) {
+                    const int k = __shfl_sync(kFull, my_slot, q);
+                    if (f < T.q[t]) bpr_slot_grad(T.p[t], T.ld[t], users, pos, neg, batch, scratch, g, lam, k, f, acc);
+                }
+            } else {
+                for (int k0 = e; k0 < n3; k0 += 32) {
+                    const int kk = k0 + lane;
+                    unsigned hits = __ballot_sync(kFull, kk < n3 && slot_id(users, pos, neg, batch, kk) == id);
+                    while (hits) {
+                        const int k = k0 + __ffs(hits) - 1;
+                        hits &= hits - 1;
+                        if (f < T.q[t]) bpr_slot_grad(T.p[t], T.ld[t], users, pos, neg, batch, scratch, g, lam, k, f, acc);
+                    }
+                }
+            }
+            if (f < T.q[t]) {
+                float4* gp = reinterpret_cast<float4*>(G.p[t] + id * G.ld[t] + f * 4);
+                float4 v = *gp;
+                v.x += acc.x; v.y += acc.y; v.z += acc.z; v.w += acc.w;
+                *gp = v;
+            }
         }
     }
 }
@@ -282,7 +330,10 @@ __global__ void __launch_bounds__(128) transr_bwd_kernel(const float* __restrict
                                                          const int64_t* __restrict__ nt, int batch, float reg,
                                                          float* __restrict__ scratch, const float* __restrict__ g_loss,
                                                          float* __restrict__ g_emb, float* __restrict__ g_rel,
-                                                         float* __restrict__ g_W, const int32_t* __restrict__ row_slot) {
+                                                         float* __restrict__ g_W, const int32_t* __restrict__ row_slot,
+                                                         float* __restrict__ work = nullptr) {
+    // work != nullptr: no atomics -- the sample's projection gradients go to work[b] (g_xh, g_xp, g_xn, g_er; K each) and its
+    // embedding gradients to its own compact rows b, B + b, 2B + b of g_emb; transr_reduce_kernel sums both in sample order
     constexpr int D = DM * 32, K = KM * 32;
     constexpr int JW = D / kTrWarps;
     __shared__ float part[kTrWarps][3][K];
@@ -333,7 +384,20 @@ __global__ void __launch_bounds__(128) transr_bwd_kernel(const float* __restrict
         gxn[m] = -gdn + lam * xn[m];
         ger[m] = gdp + gdn + lam * er[m];
     }
-    if (warp == 0) red_cols<KM>(g_rel + r * K, lane, ger);
+    if (work != nullptr) {
+        if (warp == 0) {
+            float* wb = work + (int64_t)b * 4 * K + KM * lane;
+#pragma unroll
+            for (int m = 0; m < KM; ++m) {
+                wb[m] = gxh[m];
+                wb[K + m] = gxp[m];
+                wb[2 * K + m] = gxn[m];
+                wb[3 * K + m] = ger[m];
+            }
+        }
+    } else if (warp == 0) {
+        red_cols<KM>(g_rel + r * K, lane, ger);
+    }
     // this warp's rows of W_r: d e[j] = <g_x, W_r[j, :]>, d W_r[j, :] += e[j] * g_x
     const int j0 = warp * JW;
     float* gWr = g_W + r * (int64_t)D * K;
@@ -354,7 +418,7 @@ __global__ void __launch_bounds__(128) transr_bwd_kernel(const float* __restrict
             pn = fmaf(gxn[m], w[m], pn);
             gw[m] = a * gxh[m] + bb * gxp[m] + c * gxn[m];
         }
-        red_cols<KM>(gWr + j * K, lane, gw);
+        if (work == nullptr) red_cols<KM>(gWr + j * K, lane, gw);
         ph = warp_sum(ph);
         pp = warp_sum(pp);
         pn = warp_sum(pn);
@@ -364,13 +428,121 @@ __global__ void __launch_bounds__(128) transr_bwd_kernel(const float* __restrict
             gen = pn;
         }
     }
-    if (lane < JW) {
+    if (lane < JW && work != nullptr) {
+        g_emb[(int64_t)b * D + j0 + lane] = geh;
+        g_emb[(int64_t)(batch + b) * D + j0 + lane] = gep;
+        g_emb[(int64_t)(2 * batch + b) * D + j0 + lane] = gen;
+    } else if (lane < JW) {
         // dense gradient table indexed by node, or compact rows indexed through row_slot (kgat_transr_claim_rows)
         const int64_t gh = row_slot ? row_slot[h] : h, gp = row_slot ? row_slot[p] : p, gn = row_slot ? row_slot[n] : n;
         atomicAdd(g_emb + gh * D + j0 + lane, geh);
         atomicAdd(g_emb + gp * D + j0 + lane, gep);
         atomicAdd(g_emb + gn * D + j0 + lane, gen);
     }
+}
+
+// Second pass of the deterministic TransR backward (transr_bwd_kernel with `work`), every sum in a fixed order:
+//  * blocks [0, B * D / JB): block (b, jb) -- if sample b is the first of its relation r -- adds the relation's samples' outer
+//    products e^T g_x to rows [JB jb, JB jb + JB) of g_W[r], and block (b, 0) their g_er to g_rel[r].  Warp w takes the samples
+//    i = b + w (mod kRdWarps) in increasing order; the warps' partial sums are combined in warp order;
+//  * the other blocks: one warp per id slot e; the slot that owns its node's compact row (row_slot[node] == e) replaces that
+//    row by the sum of the rows of every slot holding the node, in slot order.
+constexpr int kRdWarps = 8;
+// rows of g_W[r] per block: the warps' partial sums of the block's JB x K tile plus g_er stay inside 48 KB of shared memory
+__host__ __device__ constexpr int transr_reduce_rows(int d) { return d >= 128 ? 8 : 16; }
+template <int DM, int KM>
+__global__ void __launch_bounds__(kRdWarps * 32) transr_reduce_kernel(const float* __restrict__ emb, const int64_t* __restrict__ heads,
+                                                                     const int64_t* __restrict__ rels, const int64_t* __restrict__ pt,
+                                                                     const int64_t* __restrict__ nt, int batch, const float* __restrict__ work,
+                                                                     const int32_t* __restrict__ row_slot, float* __restrict__ g_rows,
+                                                                     float* __restrict__ g_rel, float* __restrict__ g_W) {
+    constexpr int D = DM * 32, K = KM * 32, JB = transr_reduce_rows(DM * 32), NJB = D / JB, NOUT = JB * K + K;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    int blk = blockIdx.x;
+    if (blk < batch * NJB) {
+        __shared__ float s_part[kRdWarps][NOUT];
+        const int b = blk / NJB, jb = blk % NJB, j0 = jb * JB;
+        const int64_t r = rels[b];
+        int dup = 0;
+        for (int i = tid; i < b; i += kRdWarps * 32) dup |= rels[i] == r;
+        if (__syncthreads_or(dup)) return;
+        float acc[JB][KM], acc_r[KM];
+#pragma unroll
+        for (int m = 0; m < KM; ++m) {
+            acc_r[m] = 0.f;
+#pragma unroll
+            for (int jj = 0; jj < JB; ++jj) acc[jj][m] = 0.f;
+        }
+        for (int base = b + warp; base < batch; base += kRdWarps * 32) {
+            const int il = base + kRdWarps * lane;
+            const bool mine = il < batch && rels[il] == r;
+            long long hl = 0, pl = 0, nl = 0;
+            if (mine) {
+                hl = heads[il];
+                pl = pt[il];
+                nl = nt[il];
+            }
+            unsigned hits = __ballot_sync(kFull, mine);
+            while (hits) {
+                const int src = __ffs(hits) - 1;
+                hits &= hits - 1;
+                const int i = base + kRdWarps * src;
+                const long long h = __shfl_sync(kFull, hl, src), p = __shfl_sync(kFull, pl, src), n = __shfl_sync(kFull, nl, src);
+                const float* wi = work + (int64_t)i * 4 * K + KM * lane;
+                float ehv[JB], epv[JB], env[JB];
+#pragma unroll
+                for (int c = 0; c < JB; c += 4) {
+                    const float4 a = ldg4(emb + h * D + j0 + c), bq = ldg4(emb + p * D + j0 + c), cq = ldg4(emb + n * D + j0 + c);
+                    ehv[c] = a.x; ehv[c + 1] = a.y; ehv[c + 2] = a.z; ehv[c + 3] = a.w;
+                    epv[c] = bq.x; epv[c + 1] = bq.y; epv[c + 2] = bq.z; epv[c + 3] = bq.w;
+                    env[c] = cq.x; env[c + 1] = cq.y; env[c + 2] = cq.z; env[c + 3] = cq.w;
+                }
+#pragma unroll
+                for (int m = 0; m < KM; ++m) {
+                    const float gh = wi[m], gp = wi[K + m], gn = wi[2 * K + m];
+#pragma unroll
+                    for (int jj = 0; jj < JB; ++jj) acc[jj][m] += ehv[jj] * gh + epv[jj] * gp + env[jj] * gn;
+                    if (jb == 0) acc_r[m] += wi[3 * K + m];
+                }
+            }
+        }
+#pragma unroll
+        for (int m = 0; m < KM; ++m) {
+#pragma unroll
+            for (int jj = 0; jj < JB; ++jj) s_part[warp][jj * K + KM * lane + m] = acc[jj][m];
+            s_part[warp][JB * K + KM * lane + m] = acc_r[m];
+        }
+        __syncthreads();
+        float* gWr = g_W + r * (int64_t)D * K;
+        for (int o = tid; o < NOUT; o += kRdWarps * 32) {
+            float sum = 0.f;
+#pragma unroll
+            for (int w = 0; w < kRdWarps; ++w) sum += s_part[w][o];
+            if (o < JB * K) gWr[(int64_t)(j0 + o / K) * K + o % K] += sum;
+            else if (jb == 0) g_rel[r * K + (o - JB * K)] += sum;
+        }
+        return;
+    }
+    blk -= batch * NJB;
+    const int n3 = 3 * batch, e = blk * kRdWarps + warp;
+    if (e >= n3) return;
+    const int64_t id = slot_id(heads, pt, nt, batch, e);
+    if (row_slot[id] != e) return;
+    float acc[DM];
+#pragma unroll
+    for (int c = 0; c < DM; ++c) acc[c] = 0.f;
+    for (int k0 = 0; k0 < n3; k0 += 32) {
+        const int kk = k0 + lane;
+        unsigned hits = __ballot_sync(kFull, kk < n3 && slot_id(heads, pt, nt, batch, kk) == id);
+        while (hits) {
+            const int k = k0 + __ffs(hits) - 1;
+            hits &= hits - 1;
+#pragma unroll
+            for (int c = 0; c < DM; ++c) acc[c] += g_rows[(int64_t)k * D + lane + 32 * c];
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < DM; ++c) g_rows[(int64_t)e * D + lane + 32 * c] = acc[c];
 }
 
 // Compact gradient rows for the embedding table: the 3B ids of a batch claim a slot per DISTINCT node
@@ -492,7 +664,7 @@ int kgat_bpr_backward(const kgat_tables_t* tables, const kgat_grad_tables_t* gra
         G.p[i] = grads->tables[i];
         G.ld[i] = grads->lds[i];
     }
-    bpr_bwd_kernel<<<(batch * 32 + 255) / 256, 256, 0, stream>>>(T, G, users, pos, neg, batch, reg, margin, g_loss);
+    bpr_bwd_kernel<<<(3 * batch * 32 + 255) / 256, 256, 0, stream>>>(T, G, users, pos, neg, batch, reg, margin, g_loss);
     return check_launch();
 }
 
@@ -540,9 +712,14 @@ int kgat_transr_step(const float* emb, const float* rel_emb, const float* W, int
                                                                  reinterpret_cast<float4*>(g_rows), reinterpret_cast<float4*>(g_rel_emb),
                                                                  n_rel4, reinterpret_cast<float4*>(g_W), n_w4);
     const unsigned blocks = (unsigned)batch;
+    // margin[0, 2B): per-sample margin and L2 term; margin[2B, 2B + 4BK): the deterministic backward's work rows
+    float* work = margin + 2 * batch;
+    const unsigned reduce_blocks = (unsigned)(batch * (d / transr_reduce_rows(d)) + (3 * batch + kRdWarps - 1) / kRdWarps);
     KGAT_TRANSR_DISPATCH((transr_bwd_kernel<DM, KM, true><<<blocks, 128, 0, stream>>>(emb, rel_emb, W, heads, rels, pos_tails, neg_tails,
                                                                                      batch, reg, margin, nullptr, g_rows, g_rel_emb, g_W,
-                                                                                     row_slot)));
+                                                                                     row_slot, work),
+                          transr_reduce_kernel<DM, KM><<<reduce_blocks, kRdWarps * 32, 0, stream>>>(emb, heads, rels, pos_tails, neg_tails, batch, work,
+                                                                                          row_slot, g_rows, g_rel_emb, g_W)));
     loss_reduce_kernel<<<1, 256, 0, stream>>>(margin, batch, reg, loss, loss_sum, make_publish(publish));
     return check_launch();
 }
@@ -556,9 +733,14 @@ int kgat_transr_step_claimed(const float* emb, const float* rel_emb, const float
     cudaStream_t stream = (cudaStream_t)stream_;
     if (batch <= 0 || d <= 0 || !row_slot || !g_rows || !g_rel_emb || !g_W || !loss || !margin) return KGAT_ERR_INVALID_ARGUMENT;
     const unsigned blocks = (unsigned)batch;
+    // margin[0, 2B): per-sample margin and L2 term; margin[2B, 2B + 4BK): the deterministic backward's work rows
+    float* work = margin + 2 * batch;
+    const unsigned reduce_blocks = (unsigned)(batch * (d / transr_reduce_rows(d)) + (3 * batch + kRdWarps - 1) / kRdWarps);
     KGAT_TRANSR_DISPATCH((transr_bwd_kernel<DM, KM, true><<<blocks, 128, 0, stream>>>(emb, rel_emb, W, heads, rels, pos_tails, neg_tails,
                                                                                      batch, reg, margin, nullptr, g_rows, g_rel_emb, g_W,
-                                                                                     row_slot)));
+                                                                                     row_slot, work),
+                          transr_reduce_kernel<DM, KM><<<reduce_blocks, kRdWarps * 32, 0, stream>>>(emb, heads, rels, pos_tails, neg_tails, batch, work,
+                                                                                          row_slot, g_rows, g_rel_emb, g_W)));
     loss_reduce_kernel<<<1, 256, 0, stream>>>(margin, batch, reg, loss, loss_sum, make_publish(publish));
     return check_launch();
 }

@@ -116,7 +116,7 @@ class TrainEngine:
         self.kg_loss_sum = torch.zeros(1, dtype=f32, device=dev)
         self.one = torch.ones(1, dtype=f32, device=dev)
         self.cf_scratch = torch.empty(2 * cf_batch, dtype=f32, device=dev)
-        self.kg_scratch = torch.empty(2 * kg_batch, dtype=f32, device=dev)
+        self.kg_scratch = torch.empty(ops.transr_scratch_numel(kg_batch, self.kg_params[1].shape[1]), dtype=f32, device=dev)
         self.kg_grads = [torch.zeros_like(p) for p in self.kg_params]
         # KG phase: the embedding-table gradient of a TransR batch lives in <= 3B compact rows (one slot per distinct
         # node, csrc/losses.cu: transr_claim_rows) instead of a zero-filled N x d table that Adam would re-read

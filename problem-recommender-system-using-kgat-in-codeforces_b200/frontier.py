@@ -42,9 +42,10 @@ class Frontier:
         self.counts = torch.zeros(self.n_layers, dtype=torch.int32, device=dev)
         self.scratch = torch.zeros(ops.frontier_scratch_ints(self.n), dtype=torch.int32, device=dev)
         self.bad_ids = torch.zeros(1, dtype=torch.int32, device=dev)  # ids outside [0, n) seen so far (skipped)
-        # backward of the upper (sparse) layers: scatter the edges of the few source rows (fp32 vector reductions) instead of
-        # gathering over every destination row; False = the deterministic masked gather everywhere
-        self.scatter_backward = True
+        # backward of the upper (sparse) layers: True = scatter the edges of the few source rows (fp32 vector reductions, summed
+        # in arrival order) instead of gathering over every destination row; False = the masked gather everywhere, whose fixed
+        # summation order keeps training bit-identical from run to run
+        self.scatter_backward = False
         self.serial = 0  # bumped by every user that (re)builds it, so a late backward can tell its levels were overwritten
 
     # level l in 1 .. L

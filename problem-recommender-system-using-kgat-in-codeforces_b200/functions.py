@@ -275,7 +275,7 @@ class GraphedStep:
         self.loss = torch.zeros(1, dtype=f32, device=dev)
         self.loss_scalar = self.loss.reshape(())
         self.g_loss = torch.ones(1, dtype=f32, device=dev)  # the unit upstream gradient the captured backward uses
-        self.scratch = torch.empty(2 * batch, dtype=f32, device=dev)
+        self.scratch = torch.empty(ops.transr_scratch_numel(batch, params[0].shape[-1]), dtype=f32, device=dev)
         self.counter = torch.zeros(1, dtype=torch.int64, device=dev)  # forward calls so far (dropout stream)
         self.pub_serial = torch.zeros(1, dtype=torch.int64, device=dev)  # losses published so far (device side)
         self.ring = torch.zeros(self.RING, dtype=torch.int64).pin_memory()  # (serial << 32) | float bits, written by the GPU

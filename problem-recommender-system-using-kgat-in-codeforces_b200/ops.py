@@ -479,13 +479,19 @@ def transr_claim_rows(heads, pos_t, neg_t, d: int, row_slot, g_rows):
                                      _ptr(g_rows, f32), _stream()), "transr_claim_rows")
 
 
+def transr_scratch_numel(batch: int, k: int) -> int:
+    """Floats of the ``scratch`` a fused TransR step needs: the per-sample margin and L2 term, then the per-sample projection
+    gradients its second launch reduces in sample order (bit-identical gradients from run to run)."""
+    return 2 * batch + 4 * batch * k
+
+
 @_timed("transr_step")
 def transr_step(emb, rel_emb, W, heads, rels, pos_t, neg_t, reg, loss, loss_sum, scratch, row_slot, g_rows, g_rel, g_W, publish=None):
     """Claim compact gradient rows + zero the gradient buffers, TransR forward and backward in one pass, loss value
-    (added to ``loss_sum`` when given): the KG half-step of the epoch engine in three launches."""
+    (added to ``loss_sum`` when given): the KG half-step of the epoch engine in four launches."""
     lib = _lib.load()
-    if g_rows.numel() < 3 * heads.numel() * emb.shape[1] or scratch.numel() < 2 * heads.numel():
-        raise KgatLibraryError("transr_step: g_rows needs 3 * batch * d floats, scratch 2 * batch")
+    if g_rows.numel() < 3 * heads.numel() * emb.shape[1] or scratch.numel() < transr_scratch_numel(heads.numel(), rel_emb.shape[1]):
+        raise KgatLibraryError("transr_step: g_rows needs 3 * batch * d floats, scratch transr_scratch_numel(batch, k)")
     check(lib.kgat_transr_step(_ptr(emb, f32), _ptr(rel_emb, f32), _ptr(W, f32), emb.shape[1], rel_emb.shape[1], rel_emb.shape[0],
                                _ptr(heads, i64), _ptr(rels, i64), _ptr(pos_t, i64), _ptr(neg_t, i64), heads.numel(), float(reg),
                                _ptr(loss, f32), _ptr(loss_sum, f32) if loss_sum is not None else None, _ptr(scratch, f32),
@@ -734,8 +740,8 @@ def adam_rolling_prepare(heads, pos_t, neg_t, row_slot, g_rows, zero_a, zero_b, 
 def transr_step_claimed(emb, rel_emb, W, heads, rels, pos_t, neg_t, reg, loss, loss_sum, scratch, row_slot, g_rows, g_rel, g_W, publish=None):
     """``transr_step`` for rows claimed (and buffers zeroed) by ``adam_rolling_prepare``."""
     lib = _lib.load()
-    if g_rows.numel() < 3 * heads.numel() * emb.shape[1] or scratch.numel() < 2 * heads.numel():
-        raise KgatLibraryError("transr_step_claimed: g_rows needs 3 * batch * d floats, scratch 2 * batch")
+    if g_rows.numel() < 3 * heads.numel() * emb.shape[1] or scratch.numel() < transr_scratch_numel(heads.numel(), rel_emb.shape[1]):
+        raise KgatLibraryError("transr_step_claimed: g_rows needs 3 * batch * d floats, scratch transr_scratch_numel(batch, k)")
     check(lib.kgat_transr_step_claimed(_ptr(emb, f32), _ptr(rel_emb, f32), _ptr(W, f32), emb.shape[1], rel_emb.shape[1], _ptr(heads, i64),
                                        _ptr(rels, i64), _ptr(pos_t, i64), _ptr(neg_t, i64), heads.numel(), float(reg), _ptr(loss, f32),
                                        _ptr(loss_sum, f32) if loss_sum is not None else None, _ptr(scratch, f32), _ptr(row_slot, i32),

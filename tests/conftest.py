@@ -3,7 +3,8 @@
 * registers the ``gpu`` marker (tests that need a B200 are ``@pytest.mark.gpu``),
 * puts the repo root on ``sys.path`` so ``kgat_b200`` (alias of the hyphen-named package
   directory) and ``oracle`` import,
-* loads the golden vectors produced by ``oracle/make_golden.py`` from the unmodified reference.
+* loads the golden vectors produced by ``oracle/make_golden.py`` from the unmodified reference
+  (stored as ``oracle/golden_io.py`` describes).
 """
 
 from __future__ import annotations
@@ -20,6 +21,8 @@ ROOT = Path(__file__).resolve().parents[1]
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
 
+from oracle import golden_io  # noqa: E402
+
 GOLDEN = ROOT / "tests" / "golden"
 
 
@@ -31,20 +34,24 @@ class Golden:
     """A golden ``.npz`` with helpers to rebuild reference-shaped objects."""
 
     def __init__(self, name: str):
-        self.z = np.load(GOLDEN / name, allow_pickle=False)
+        self.z = golden_io.load(GOLDEN / name)
 
     def __getitem__(self, k):
         return self.z[k]
 
     def __contains__(self, k):
-        return k in self.z.files
+        return k in self.z
 
     def keys(self):
-        return self.z.files
+        return list(self.z)
+
+    def cut(self, k, full):
+        """A computed output restricted to the rows the golden stores of ``k`` (all of them unless ``k`` is a row sample)."""
+        return golden_io.cut(self.z, k, full)
 
     def params(self, prefix: str = "param::", device="cpu") -> "OrderedDict[str, torch.Tensor]":
         out = OrderedDict()
-        for k in self.z.files:
+        for k in self.z:
             if k.startswith(prefix):
                 out[k[len(prefix) :]] = torch.from_numpy(self.z[k].copy()).to(device)
         return out

@@ -259,8 +259,8 @@ def test_pruned_cf_step_equals_full_propagation(kb, layer_size, mode):
 
     g, model = _small_model(kb, layer_size)
     model.api_graphs = False
-    if mode == "eval-gather":
-        model._frontier(model.cuda()._graph(), 3 * 6).scatter_backward = False
+    if mode in ("eval", "eval-gather"):  # the edge scatter is no longer the default: select each backward explicitly
+        model._frontier(model.cuda()._graph(), 3 * 6).scatter_backward = mode == "eval"
         mode = "eval"
     rng = np.random.default_rng(len(layer_size))
     b = 6
