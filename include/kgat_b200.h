@@ -32,7 +32,7 @@ extern "C" {
 #define KGAT_ERR_UNSUPPORTED (-3)
 #define KGAT_ERR_WORKSPACE (-4)
 
-#define KGAT_ABI_VERSION 9
+#define KGAT_ABI_VERSION 10
 #define KGAT_MAX_LAYERS 8   /* embedding table + up to 7 propagation layers */
 #define KGAT_MAX_TENSORS 24 /* tensors per multi-tensor Adam launch */
 #define KGAT_MAX_PEERS 31   /* other ranks of a row-sharded propagation */
@@ -358,7 +358,33 @@ int kgat_topk_rows(const float* scores, int64_t ld, int32_t m, int32_t n, int32_
                    float* val_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
-/* K11: Adam                                 reference model.py:393-419 (torch.optim.Adam)       */
+/* Path explanations: why a problem reaches a user through A (no counterpart in the reference,     */
+/* whose --visualize_attention / weights_visualizer.py:19 read single entries attentive_matrix[u,p]) */
+/* ------------------------------------------------------------------------------------------- */
+/* For each of n_pairs pairs (src[j], dst[j]) of node ids (int32, e.g. from kgat_ids64_to_i32): the simple paths
+ * s = v0 -> v1 -> ... -> vh = t of 1 <= h <= max_hops (max_hops in {1, 2, 3}) hops whose every hop (v_m, v_m+1) is a
+ * stored entry of A (a column of CSR row v_m; the direction of propagation, so the path carries t's embedding into s).
+ * Weight = fp32 product of the hop values left to right, ((A[v0,v1] * A[v1,v2]) * A[v2,v3]).  Paths rank by weight
+ * descending, then h ascending, then (v1, v2) ascending.  s == t, or an id outside [0, n_nodes), has no paths.
+ * A: CSR (row_ptr, col_idx, vals) with sorted unique columns per row, and its transpose (t_ptr, t_idx) with t_perm mapping
+ * a transposed slot to its CSR slot (graph.py: AttentiveGraph).  k in [1, 64].  Outputs (P = n_pairs, H = max_hops):
+ *   nodes  int64 [P, k, H+1]  v0..vh, -1 after vh and for missing paths
+ *   slots  int64 [P, k, H]    CSR slot of every hop (= index into the COO view's indices / values), -1 padding
+ *   hops   int32 [P, k]       h, 0 for a missing path
+ *   weight fp32  [P, k]       path weight, 0 for a missing path
+ *   count  int64 [P, H]       number of simple paths of each length
+ *   mass   fp32  [P, H]       their summed weight (fp64 sums in a fixed order: bitwise reproducible)
+ * Work per pair is sum over the intersections (row s & In t, row a & In t for a in row s) of the shorter list times
+ * log of the longer; it is spread over several CTAs per pair.  Two launches, no host synchronisation; workspace
+ * size from kgat_explain_paths_workspace_bytes (depends on n_pairs and k only; -1 for invalid arguments). */
+int64_t kgat_explain_paths_workspace_bytes(int64_t n_pairs, int32_t k, int32_t max_hops);
+int kgat_explain_paths(const int32_t* row_ptr, const int32_t* col_idx, const float* vals, const int32_t* t_ptr, const int32_t* t_idx,
+                       const int32_t* t_perm, int64_t n_nodes, const int32_t* src, const int32_t* dst, int64_t n_pairs, int32_t k,
+                       int32_t max_hops, int64_t* nodes, int64_t* slots, int32_t* hops, float* weight, int64_t* count, float* mass,
+                       void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------- */
+/* K11: Adam                               reference model.py:393-419 (torch.optim.Adam)       */
 /* ------------------------------------------------------------------------------------------- */
 typedef struct {
     int32_t n_tensors;

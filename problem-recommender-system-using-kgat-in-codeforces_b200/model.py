@@ -52,6 +52,20 @@ class KGATArgs:
     regularization_params: list[float] = field(default_factory=lambda: [1e-5, 1e-5])
 
 
+@dataclass
+class PathExplanation:
+    """Result of ``KGAT.explain`` for P (user, item) pairs, k paths each, up to H hops (see ``ops.explain_paths``).
+    A slot indexes ``attentive_matrix.indices()`` / ``.values()``; missing paths and positions after the last hop hold -1
+    (``hops`` 0, ``weight`` 0)."""
+
+    nodes: torch.Tensor  # int64 [P, k, H+1]: user node, intermediate nodes, item node
+    slots: torch.Tensor  # int64 [P, k, H]
+    hops: torch.Tensor  # int32 [P, k]
+    weight: torch.Tensor  # fp32 [P, k]: product of the hop values
+    count: torch.Tensor  # int64 [P, H]: number of paths of each length
+    mass: torch.Tensor  # fp32 [P, H]: summed weight of those paths
+
+
 class KGATMode(IntEnum):
     TRAIN_CF = 0
     TRAIN_KG = 1
@@ -573,6 +587,36 @@ class KGAT(nn.Module):
         if mask_ptr is not None:
             ops.mask_scores_(scores, mask_ptr, mask_items)
         return ops.topk_rows(scores, k, want_values)
+
+    @torch.no_grad()
+    def explain(self, user_ids, item_ids, k: int = 10, max_hops: int | None = None) -> "PathExplanation":
+        """Why item ``item_ids[j]`` reaches user ``user_ids[j]``: the top-``k`` simple paths of 1 .. ``max_hops`` hops from the
+        user's CKG node to the item's CKG node ``user_num + item`` through the current ``attentive_matrix`` A, ranked by the
+        product of their attention values (weight descending, then fewer hops, then lower (v1, v2)), with the number and
+        summed weight of all such paths per length.  A hop (v, w) is a stored entry A[v, w]: the direction in which
+        propagation carries w's embedding into v.
+
+        ``max_hops`` defaults to ``min(3, number of layers)``.  Ids: int32 / int64, CPU or CUDA; users in
+        ``[0, user_num)``, items in ``[0, entity_num)``.
+
+        Unlike PREDICT, which scores problem ``p`` from row ``p`` of the propagated table (quirk Q4, reproduced on purpose,
+        SURVEY.md), the paths end at the problem's own CKG node ``user_num + p``, the node the graph links to its solvers,
+        contest, tags and rating.
+
+        Reads only the attentive matrix: it does not settle deferred KG rows, invalidate caches or captured steps, or draw
+        from torch's RNG, so calling it between training steps leaves training unchanged."""
+        max_hops = min(3, self._layer_num) if max_hops is None else int(max_hops)
+        users, items = self._ids(user_ids).flatten(), self._ids(item_ids).flatten()
+        if users.numel() != items.numel():
+            raise ValueError(f"user_ids and item_ids differ in length ({users.numel()} != {items.numel()})")
+        if users.numel():
+            lo_u, hi_u, lo_i, hi_i = torch.stack([users.min(), users.max(), items.min(), items.max()]).tolist()
+            if lo_u < 0 or hi_u >= self._user_num:
+                raise ValueError(f"user ids must lie in [0, {self._user_num})")
+            if lo_i < 0 or hi_i >= self._entity_num:
+                raise ValueError(f"item ids must lie in [0, {self._entity_num})")
+        nodes, slots, hops, weight, count, mass = ops.explain_paths(self._graph(), users, items + self._user_num, k, max_hops)
+        return PathExplanation(nodes=nodes, slots=slots, hops=hops, weight=weight, count=count, mass=mass)
 
     # ------------------------------------------------------------------------------------------
     # A10: optimisers

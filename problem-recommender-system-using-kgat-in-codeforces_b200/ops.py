@@ -676,6 +676,46 @@ def topk_rows(scores, k: int, want_values: bool = False):
     return (idx, val) if want_values else idx
 
 
+def explain_paths(graph, src: torch.Tensor, dst: torch.Tensor, k: int, max_hops: int):
+    """Top-``k`` attention-weighted simple paths of 1 .. ``max_hops`` hops from ``src[j]`` to ``dst[j]`` through the attentive
+    matrix of ``graph`` (an ``AttentiveGraph``), with the number and summed weight of all such paths per length
+    (``kgat_explain_paths``).  ``src`` / ``dst``: node ids, any integer dtype, on the graph's device.
+    Returns ``(nodes [P,k,H+1] int64, slots [P,k,H] int64, hops [P,k] int32, weight [P,k] fp32, count [P,H] int64,
+    mass [P,H] fp32)``.  Raises ``ValueError`` for an id outside ``[0, graph.n)`` (read back after the launches)."""
+    k, max_hops = int(k), int(max_hops)
+    if not 1 <= k <= 64:
+        raise ValueError(f"k must be in [1, 64], got {k}")
+    if max_hops not in (1, 2, 3):
+        raise ValueError(f"max_hops must be 1, 2 or 3, got {max_hops}")
+    if src.dim() != 1 or dst.dim() != 1 or src.numel() != dst.numel():
+        raise ValueError(f"src and dst must be 1-D of equal length, got {tuple(src.shape)} and {tuple(dst.shape)}")
+    lib = _lib.load()
+    dev = graph.col_idx.device
+    P, H = src.numel(), max_hops
+    nodes = torch.empty(P, k, H + 1, dtype=i64, device=dev)
+    slots = torch.empty(P, k, H, dtype=i64, device=dev)
+    hops = torch.empty(P, k, dtype=i32, device=dev)
+    weight = torch.empty(P, k, dtype=f32, device=dev)
+    count = torch.empty(P, H, dtype=i64, device=dev)
+    mass = torch.empty(P, H, dtype=f32, device=dev)
+    if P == 0:
+        return nodes, slots, hops, weight, count, mass
+    ids = torch.cat([src.to(device=dev, dtype=i64), dst.to(device=dev, dtype=i64)]).contiguous()
+    ids32 = torch.empty(2 * P, dtype=i32, device=dev)
+    bad = torch.zeros(1, dtype=i32, device=dev)
+    check(lib.kgat_ids64_to_i32(_ptr(ids, i64), 2 * P, graph.n, ids32.data_ptr(), bad.data_ptr(), _stream()), "explain_paths ids")
+    ws_bytes = int(lib.kgat_explain_paths_workspace_bytes(P, k, H))
+    ws = torch.empty(max(ws_bytes, 1), dtype=u8, device=dev)
+    check(lib.kgat_explain_paths(
+        _ptr(graph.row_ptr, i32), _ptr(graph.col_idx, i32), _ptr(graph.vals, f32), _ptr(graph.t_ptr, i32), _ptr(graph.t_idx, i32),
+        _ptr(graph.t_perm, i32), graph.n, ids32.data_ptr(), ids32.data_ptr() + 4 * P, P, k, H, nodes.data_ptr(), slots.data_ptr(),
+        hops.data_ptr(), weight.data_ptr(), count.data_ptr(), mass.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "explain_paths")
+    n_bad = int(bad.item())
+    if n_bad:
+        raise ValueError(f"{n_bad} node id(s) outside [0, {graph.n})")
+    return nodes, slots, hops, weight, count, mass
+
+
 # ----------------------------------------------------------------------------------------------
 # K11 Adam
 # ----------------------------------------------------------------------------------------------
