@@ -32,7 +32,7 @@ extern "C" {
 #define KGAT_ERR_UNSUPPORTED (-3)
 #define KGAT_ERR_WORKSPACE (-4)
 
-#define KGAT_ABI_VERSION 10
+#define KGAT_ABI_VERSION 11
 #define KGAT_MAX_LAYERS 8   /* embedding table + up to 7 propagation layers */
 #define KGAT_MAX_TENSORS 24 /* tensors per multi-tensor Adam launch */
 #define KGAT_MAX_PEERS 31   /* other ranks of a row-sharded propagation */
@@ -382,6 +382,36 @@ int kgat_explain_paths(const int32_t* row_ptr, const int32_t* col_idx, const flo
                        const int32_t* t_perm, int64_t n_nodes, const int32_t* src, const int32_t* dst, int64_t n_pairs, int32_t k,
                        int32_t max_hops, int64_t* nodes, int64_t* slots, int32_t* hops, float* weight, int64_t* count, float* mass,
                        void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------- */
+/* Filtered top-k recommendations for many users in one call (the reference's recommend(),        */
+/* main.py:541-636, loops over 256-user batches of a materialised score matrix)                   */
+/* ------------------------------------------------------------------------------------------- */
+/* Candidate filter.  Item items[i] (int32, in [0, n_nodes - user_num)) passes iff, for every group g < n_groups, CSR row
+ * user_num + items[i] of A (sorted unique columns) stores a column among group_nodes[group_ptr[g] .. group_ptr[g+1]) (node
+ * ids; a stored entry counts whatever its value).  n_groups = 0 passes every item.  Outputs, in input order: positions[j] =
+ * index into items of the j-th passing item, cand_items[j] = items[positions[j]] (both n_items int32; `positions` is also
+ * the scratch of the flags), *n_cand = their number (device int32).  Two launches, no host synchronisation. */
+int kgat_recommend_filter(const int32_t* row_ptr, const int32_t* col_idx, int64_t n_nodes, int32_t user_num, const int32_t* items,
+                          int64_t n_items, const int32_t* group_ptr, const int32_t* group_nodes, int32_t n_groups, int32_t* positions,
+                          int32_t* cand_items, int32_t* n_cand, void* stream);
+/* Top-k candidates per user without materialising scores.  users[b]: table rows (int32); candidates: cand_items[0 .. n)
+ * (int32 table rows, unique), n = *n_cand when n_cand != NULL (e.g. from kgat_recommend_filter) else n_cand_max.
+ * Score(b, c) = sequential fp32 fmaf chain over the concatenated row of the tables from +0 (zero columns padded to a multiple
+ * of 16), exactly kgat_gather_concat + kgat_sgemm_nt.  exclude_ptr / exclude_items (nullable): CSR over table rows of users,
+ * items ascending per user; candidate c is skipped for user b when cand_items[c] is in users[b]'s list.  Order: descending
+ * key of kgat_topk_rows (NaN largest, -0 below +0), then lower candidate index.  k in [1, 128]; slices in [0, 64] = candidate
+ * slices per 64-user tile (0 = chosen from n_users, the SM count and the CTAs per SM; the result does not depend on it).  Outputs:
+ *   out_items  int64 [n_users, k]  cand_items of the ranked candidates, -1 after out_count[b]
+ *   out_scores fp32  [n_users, k]  their scores, -inf after out_count[b]
+ *   out_count  int32 [n_users]     min(k, number of candidates not excluded for users[b])
+ * Two launches, no host synchronisation; workspace from kgat_recommend_workspace_bytes with the same arguments (-1 for
+ * invalid ones, or a row too wide for shared memory).  KGAT_ERR_UNSUPPORTED when the concatenated row is too wide for shared
+ * memory at this k. */
+int64_t kgat_recommend_workspace_bytes(const kgat_tables_t* tables, int64_t n_users, int64_t n_cand_max, int32_t k, int32_t slices);
+int kgat_recommend_topk(const kgat_tables_t* tables, const int32_t* users, int64_t n_users, const int32_t* cand_items, int64_t n_cand_max,
+                        const int32_t* n_cand, int32_t k, const int32_t* exclude_ptr, const int32_t* exclude_items, int32_t slices,
+                        int64_t* out_items, float* out_scores, int32_t* out_count, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* K11: Adam                               reference model.py:393-419 (torch.optim.Adam)       */

@@ -13,7 +13,7 @@ from pathlib import Path
 
 KGAT_MAX_LAYERS = 8
 KGAT_MAX_TENSORS = 24
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 _PKG_DIR = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ.get("KGAT_B200_LIB", _PKG_DIR / "lib" / "libkgat_b200.so"))
@@ -122,6 +122,9 @@ SIGNATURES: dict[str, tuple] = {
     "kgat_topk_rows": (_I32, [_P, _I64, _I32, _I32, _I32, _P, _P, _P]),
     "kgat_explain_paths_workspace_bytes": (_I64, [_I64, _I32, _I32]),
     "kgat_explain_paths": (_I32, [_P, _P, _P, _P, _P, _P, _I64, _P, _P, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _I64, _P]),
+    "kgat_recommend_filter": (_I32, [_P, _P, _I64, _I32, _P, _I64, _P, _P, _I32, _P, _P, _P, _P]),
+    "kgat_recommend_workspace_bytes": (_I64, [C.POINTER(TablesT), _I64, _I64, _I32, _I32]),
+    "kgat_recommend_topk": (_I32, [C.POINTER(TablesT), _P, _I64, _P, _I64, _P, _I32, _P, _P, _I32, _P, _P, _P, _P, _I64, _P]),
     "kgat_adam_advance": (_I32, [_P, _D, _D, _D, _D, _P, _P]),
     "kgat_adam_set_hyper": (_I32, [_I64, _D, _D, _D, _D, _P, _P]),
     "kgat_adam_apply": (_I32, [C.POINTER(AdamTensorsT), _P, _P]),
@@ -162,7 +165,7 @@ KERNELS_PER_CALL = {
     "kgat_frontier_list": 2, "kgat_frontier_zero_rows": 1, "kgat_frontier_segment": 1, "kgat_biagg_forward_rows": 1, "kgat_biagg_backward_rows": 1, "kgat_biagg_forward": 1, "kgat_biagg_backward": 1,
     "kgat_biagg_reduce_param_grads": 1, "kgat_bpr_forward": 2, "kgat_bpr_backward": 1, "kgat_transr_forward": 2,
     "kgat_transr_backward": 1, "kgat_att_pair_scores": 1, "kgat_mha_forward": 1, "kgat_att_pair_project": 1, "kgat_att_edge_scores_kgat": 1, "kgat_att_edge_scores_dropout": 1, "kgat_att_row_softmax": 1,
-    "kgat_att_edge_weights": 1, "kgat_gather_concat": 1, "kgat_sgemm_nt": 1, "kgat_mask_scores": 1, "kgat_topk_rows": 1, "kgat_explain_paths": 2,
+    "kgat_att_edge_weights": 1, "kgat_gather_concat": 1, "kgat_sgemm_nt": 1, "kgat_mask_scores": 1, "kgat_topk_rows": 1, "kgat_explain_paths": 2, "kgat_recommend_filter": 2, "kgat_recommend_topk": 2,
     "kgat_adam_advance": 1, "kgat_adam_set_hyper": 1, "kgat_adam_apply": 1, "kgat_adam_hyper_table": 1, "kgat_adam_lazy_catchup": 1, "kgat_adam_sparse_rows": 1,
     "kgat_adam_lazy_flush": 1, "kgat_fill_f32": 1, "kgat_select_batch_i64": 1, "kgat_sample_cf_batch": 1, "kgat_sample_kg_batch": 1,
     "kgat_peer_push": 1, "kgat_peer_push_rows": 1, "kgat_publish_loss": 1, "kgat_zero_rows_i64": 1, "kgat_transr_rows_to_dense": 1, "kgat_transr_release_rows": 1, "kgat_peer_signal_wait": 1, "kgat_transr_claim_rows": 1, "kgat_transr_step": 4,

@@ -78,6 +78,51 @@ __device__ __forceinline__ void fma4(float4& a, float s, const float4& x) {
 }
 __device__ __forceinline__ float lrelu(float z) { return z > 0.f ? z : KGAT_LEAKY_SLOPE * z; }
 
+// order-preserving map: larger float -> larger key; -inf smallest; NaN treated as largest (torch.sort)
+__device__ __forceinline__ uint32_t float_key(float f) {
+    uint32_t u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+// first position in p[0, n) whose value is >= x (p ascending)
+__device__ __forceinline__ int lower_bound_i32(const int32_t* __restrict__ p, int n, int x) {
+    int lo = 0;
+    while (n > 0) {
+        const int half = n >> 1;
+        if (__ldg(p + lo + half) < x) {
+            lo += half + 1;
+            n -= half + 1;
+        } else {
+            n = half;
+        }
+    }
+    return lo;
+}
+
+// kgat_tables_t in float4 units: table t holds columns [4 qoff[t], 4 qoff[t+1]) of the concatenated row
+struct ConcatTables {
+    int n;
+    int q[KGAT_MAX_LAYERS];
+    int qoff[KGAT_MAX_LAYERS + 1];
+    const float* p[KGAT_MAX_LAYERS];
+    int64_t ld[KGAT_MAX_LAYERS];
+};
+
+// false when a table is missing or a width / leading dimension is not a multiple of 4
+inline bool tables_from(const kgat_tables_t* t, ConcatTables* T) {
+    if (!t || t->n_tables <= 0 || t->n_tables > KGAT_MAX_LAYERS) return false;
+    T->n = t->n_tables;
+    T->qoff[0] = 0;
+    for (int i = 0; i < T->n; ++i) {
+        if (t->dims[i] <= 0 || (t->dims[i] & 3) || (t->lds[i] & 3) || !t->tables[i]) return false;
+        T->q[i] = t->dims[i] / 4;
+        T->qoff[i + 1] = T->qoff[i] + T->q[i];
+        T->p[i] = t->tables[i];
+        T->ld[i] = t->lds[i];
+    }
+    return true;
+}
+
 // log(sigmoid(x)) as ATen computes it: min(x,0) - log1p(exp(-|x|))
 __device__ __forceinline__ float log_sigmoid(float x) { return fminf(x, 0.f) - log1pf(expf(-fabsf(x))); }
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }

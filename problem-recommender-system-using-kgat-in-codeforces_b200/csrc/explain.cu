@@ -38,21 +38,6 @@ __device__ __forceinline__ bool beats(const Cand& a, const Cand& b) {
     return a.v2 < b.v2;
 }
 
-// first position in p[0, n) whose value is >= x (p ascending)
-__device__ __forceinline__ int lower_bound_i32(const int32_t* __restrict__ p, int n, int x) {
-    int lo = 0;
-    while (n > 0) {
-        const int half = n >> 1;
-        if (__ldg(p + lo + half) < x) {
-            lo += half + 1;
-            n -= half + 1;
-        } else {
-            n = half;
-        }
-    }
-    return lo;
-}
-
 int explain_units(int64_t n_pairs) {
     const int64_t u = 65536 / (n_pairs > 0 ? n_pairs : 1);
     return (int)(u < 8 ? 8 : (u > 64 ? 64 : u));

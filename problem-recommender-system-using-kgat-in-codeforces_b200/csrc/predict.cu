@@ -6,15 +6,7 @@
 namespace kgat {
 namespace {
 
-struct Tables {
-    int n;
-    int q[KGAT_MAX_LAYERS];
-    int qoff[KGAT_MAX_LAYERS + 1];
-    const float* p[KGAT_MAX_LAYERS];
-    int64_t ld[KGAT_MAX_LAYERS];
-};
-
-__global__ void __launch_bounds__(256) gather_concat_kernel(Tables T, const int64_t* __restrict__ ids, int64_t n_ids,
+__global__ void __launch_bounds__(256) gather_concat_kernel(ConcatTables T, const int64_t* __restrict__ ids, int64_t n_ids,
                                                             float* __restrict__ out, int64_t ld_out) {
     const int lane = threadIdx.x & 31;
     const int64_t b = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -83,12 +75,6 @@ __global__ void mask_scores_kernel(float* __restrict__ scores, int64_t ld, int m
         const int c = mask_items[p];
         if (c >= 0 && c < n) scores[(int64_t)row * ld + c] = -INFINITY;
     }
-}
-
-// order-preserving map: larger float -> larger key; -inf smallest; NaN treated as largest (torch.sort)
-__device__ __forceinline__ uint32_t float_key(float f) {
-    uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
 // Exact top-K of one row per CTA via 3-pass radix select on the 32-bit key, then an ordered
@@ -196,16 +182,8 @@ extern "C" {
 int kgat_gather_concat(const kgat_tables_t* t, const int64_t* ids64, int64_t n_ids, float* out, int64_t ld_out, void* stream) {
     if (!t || t->n_tables <= 0 || t->n_tables > KGAT_MAX_LAYERS || n_ids < 0 || (ld_out & 3)) return KGAT_ERR_INVALID_ARGUMENT;
     if (n_ids == 0) return KGAT_OK;
-    Tables T;
-    T.n = t->n_tables;
-    T.qoff[0] = 0;
-    for (int i = 0; i < T.n; ++i) {
-        if (t->dims[i] <= 0 || (t->dims[i] & 3) || (t->lds[i] & 3) || !t->tables[i]) return KGAT_ERR_INVALID_ARGUMENT;
-        T.q[i] = t->dims[i] / 4;
-        T.qoff[i + 1] = T.qoff[i] + T.q[i];
-        T.p[i] = t->tables[i];
-        T.ld[i] = t->lds[i];
-    }
+    ConcatTables T;
+    if (!tables_from(t, &T)) return KGAT_ERR_INVALID_ARGUMENT;
     gather_concat_kernel<<<(unsigned)((n_ids * 32 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(T, ids64, n_ids, out, ld_out);
     return check_launch();
 }

@@ -48,6 +48,16 @@ class InteractionCSR:
         self.counts = torch.from_numpy(counts.astype(np.int64)).to(device)
         users = np.repeat(np.arange(user_num, dtype=np.int64), counts)
         self.keys = torch.from_numpy(np.sort(users * item_num + flat)).to(device)  # sorted (user, item) keys
+        self._ptr_dev = None
+
+    @property
+    def ptr_dev(self) -> torch.Tensor:
+        """Row pointer over all users as int32 on the device of ``items`` (built on first use; ``KGAT.recommend`` reads it)."""
+        if self._ptr_dev is None:
+            if self.ptr_host[-1] > np.iinfo(np.int32).max:
+                raise ValueError("more than 2^31 - 1 interactions do not fit the int32 row pointer")
+            self._ptr_dev = torch.from_numpy(self.ptr_host.astype(np.int32)).to(self.items.device)
+        return self._ptr_dev
 
     def batch(self, start: int, stop: int):
         """(ptr int32 [b+1] relative to the batch, items int32) for users [start, stop)."""

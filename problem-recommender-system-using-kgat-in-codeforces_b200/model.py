@@ -66,6 +66,16 @@ class PathExplanation:
     mass: torch.Tensor  # fp32 [P, H]: summed weight of those paths
 
 
+@dataclass
+class Recommendation:
+    """Result of ``KGAT.recommend`` for U users: each user's top-k eligible problems, best first.  Positions from ``count`` on
+    hold item -1 and score -inf."""
+
+    items: torch.Tensor  # int64 [U, k]: problem ids
+    scores: torch.Tensor  # fp32 [U, k]: the PREDICT scores of those problems
+    count: torch.Tensor  # int32 [U]: min(k, number of eligible problems)
+
+
 class KGATMode(IntEnum):
     TRAIN_CF = 0
     TRAIN_KG = 1
@@ -587,6 +597,57 @@ class KGAT(nn.Module):
         if mask_ptr is not None:
             ops.mask_scores_(scores, mask_ptr, mask_items)
         return ops.topk_rows(scores, k, want_values)
+
+    @torch.no_grad()
+    def recommend(self, user_ids, items, k: int = 20, exclude=None, require=None) -> "Recommendation":
+        """Each user's top-``k`` problems among ``items``, in one call for any number of users, without a score matrix.
+
+        ``user_ids``: 1-D int32 / int64, CPU or CUDA, in ``[0, user_num)``, repeats allowed.  ``items``: an int ``n`` (= ``arange(n)``)
+        or a 1-D tensor of unique problem ids in ``[0, entity_num)``; its order breaks score ties.  ``exclude``: ``None`` or a
+        ``metrics.InteractionCSR`` over the same ``user_num`` (e.g. training positives and solved problems); problem ``p`` is not
+        recommended to ``u`` when it is in ``u``'s list.  ``require``: ``None`` or a list of non-empty groups of entity ids; ``p``
+        passes a group when the current ``attentive_matrix`` stores an entry at ``(user_num + p, user_num + e)`` for some ``e`` of
+        the group (whatever its value), and must pass every group -- e.g. ``[[rating_1600, ..., rating_1900], [tag_dp]]``.
+
+        A score is exactly the fp32 value ``model(u, p, mode=PREDICT)`` and ``recommend_topk`` give; the order is score
+        descending (NaN first, -0 after +0), then earlier position in ``items``.  ``1 <= k <= 128``; users with fewer than ``k``
+        eligible problems get ``count < k`` and -1 / -inf padding.
+
+        Like PREDICT the scores use row ``p`` of the propagated table (quirk Q4, reproduced on purpose, SURVEY.md), while the
+        filter reads the problem's own CKG node ``user_num + p``, as ``explain`` does.  Uses the cached propagation after settling
+        deferred KG rows, and honours train / eval mode as PREDICT does: call it in ``eval()``."""
+        k = int(k)
+        if not 1 <= k <= 128:
+            raise ValueError(f"k must be in [1, 128], got {k}")
+        dev = self._device()
+        users = torch.as_tensor(user_ids)
+        if users.dim() != 1 or users.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f"user_ids must be a 1-D int32 / int64 tensor, got {users.dtype} of shape {tuple(users.shape)}")
+        users = users.to(device=dev, dtype=torch.int64)
+        if isinstance(items, int):
+            if not 0 <= items <= self._entity_num:
+                raise ValueError(f"items = {items} must lie in [0, {self._entity_num}]")
+            cand = torch.arange(items, device=dev)
+        else:
+            cand = torch.as_tensor(items)
+            if cand.dim() != 1 or cand.dtype not in (torch.int32, torch.int64):
+                raise ValueError(f"items must be an int or a 1-D int32 / int64 tensor, got {cand.dtype} of shape {tuple(cand.shape)}")
+            cand = cand.to(device=dev, dtype=torch.int64)
+        if exclude is not None and exclude.user_num != self._user_num:
+            raise ValueError(f"exclude covers {exclude.user_num} users, the model has {self._user_num}")
+        if require is not None:
+            require = ops.require_groups(require, self._entity_num)
+        # ranges and duplicates in one read-back: the only host synchronisation of the call
+        dup = (torch.sort(cand).values.diff() == 0).sum() if cand.numel() > 1 else torch.zeros((), dtype=torch.int64, device=dev)
+        users32, cand32 = ops.range_check([("user ids", users, self._user_num), ("item ids", cand, self._entity_num)], dev,
+                                          flags=[("items holds duplicate ids", dup)])
+        tables = self._tables()
+        n_cand = None
+        if require is not None:
+            _, cand32, n_cand = ops.launch_recommend_filter(self._graph(), cand32, require, self._user_num)
+        ex_ptr, ex_items = (exclude.ptr_dev.to(dev), exclude.items.to(dev)) if exclude is not None else (None, None)
+        out_items, scores, count = ops.launch_recommend_topk(tables, users32, cand32, k, ex_ptr, ex_items, n_cand=n_cand)
+        return Recommendation(items=out_items, scores=scores, count=count)
 
     @torch.no_grad()
     def explain(self, user_ids, item_ids, k: int = 10, max_hops: int | None = None) -> "PathExplanation":

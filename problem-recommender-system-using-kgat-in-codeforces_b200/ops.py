@@ -716,6 +716,133 @@ def explain_paths(graph, src: torch.Tensor, dst: torch.Tensor, k: int, max_hops:
     return nodes, slots, hops, weight, count, mass
 
 
+def _ids64(ids: torch.Tensor, name: str, dev) -> torch.Tensor:
+    """1-D ids of any integer dtype, CPU or CUDA -> contiguous int64 on ``dev``."""
+    if ids.dim() != 1 or ids.dtype.is_floating_point or ids.dtype == torch.bool:
+        raise ValueError(f"{name} must be a 1-D integer tensor, got {ids.dtype} of shape {tuple(ids.shape)}")
+    return ids.to(device=dev, dtype=i64).contiguous()
+
+
+def range_check(checks, dev, flags=()) -> list:
+    """checks: (name, int64 ids on dev, bound >= 1); flags: (message, device integer scalar that is nonzero on failure).
+    Converts every id list to int32 and reads the out-of-range counts and the flags back in one synchronisation, before any
+    kernel indexes with the ids; ValueError for the first check or flag that fails.  Returns the int32 id lists."""
+    lib = _lib.load()
+    bad = torch.zeros(len(checks) + len(flags), dtype=i32, device=dev)
+    outs = []
+    for j, (name, ids, bound) in enumerate(checks):
+        out = torch.empty(ids.numel(), dtype=i32, device=dev)
+        if ids.numel():
+            check(lib.kgat_ids64_to_i32(_ptr(ids, i64), ids.numel(), bound, out.data_ptr(), bad.data_ptr() + 4 * j, _stream()), name)
+        outs.append(out)
+    for j, (_, flag) in enumerate(flags):
+        bad[len(checks) + j] = flag
+    got = bad.tolist()
+    for (name, _, bound), n_bad in zip(checks, got):
+        if n_bad:
+            raise ValueError(f"{n_bad} {name} outside [0, {bound})")
+    for (msg, _), n_bad in zip(flags, got[len(checks) :]):
+        if n_bad:
+            raise ValueError(msg)
+    return outs
+
+
+def require_groups(groups, n_ent: int):
+    """``require`` groups as lists of ints; ValueError for an empty group or an entity id outside ``[0, n_ent)``."""
+    groups = [list(map(int, g)) for g in groups]
+    if any(len(g) == 0 for g in groups):
+        raise ValueError("every group of `require` must hold at least one entity id")
+    if any(not 0 <= e < n_ent for g in groups for e in g):
+        raise ValueError(f"entity ids of `require` must lie in [0, {n_ent})")
+    return groups
+
+
+def recommend_filter(graph, items: torch.Tensor, groups, user_num: int):
+    """Candidate filter of ``KGAT.recommend`` (``kgat_recommend_filter``): keeps the items ``p`` of ``items`` (entity ids) whose
+    CKG node ``user_num + p`` has a stored entry of ``graph`` (an ``AttentiveGraph``) towards ``user_num + e`` for some ``e`` of
+    every group.  ``groups``: list of non-empty lists of entity ids in ``[0, graph.n - user_num)``.
+    Returns ``(positions int32 [len(items)], cand_items int32 [len(items)], n_cand int32 [1])``, all on the device: the first
+    ``n_cand`` entries are the passing positions into ``items`` in input order and their item ids (``cand_items`` is 0 after them)."""
+    user_num = int(user_num)
+    if not 0 <= user_num < graph.n:
+        raise ValueError(f"user_num {user_num} outside [0, {graph.n})")
+    dev = graph.col_idx.device
+    groups = require_groups(groups, graph.n - user_num)
+    (items32,) = range_check([("item ids", _ids64(items, "items", dev), graph.n - user_num)], dev)
+    return launch_recommend_filter(graph, items32, groups, user_num)
+
+
+def launch_recommend_filter(graph, items32: torch.Tensor, groups, user_num: int):
+    """``recommend_filter`` for int32 ``items32`` and ``groups`` already known to lie in range (no checks, no synchronisation)."""
+    lib = _lib.load()
+    dev = graph.col_idx.device
+    flat = [e for g in groups for e in g]
+    gptr = torch.tensor([0] + [len(g) for g in groups], dtype=i64).cumsum(0).to(dtype=i32, device=dev)
+    gnodes = torch.tensor(flat, dtype=i32).add_(user_num).to(dev)
+    n = items32.numel()
+    positions = torch.empty(n, dtype=i32, device=dev)
+    cand = torch.zeros(n, dtype=i32, device=dev)  # entries from n_cand on stay 0, a valid row for recommend_topk_fused's range check
+    n_cand = torch.empty(1, dtype=i32, device=dev)
+    check(lib.kgat_recommend_filter(_ptr(graph.row_ptr, i32), _ptr(graph.col_idx, i32), graph.n, user_num, _ptr(items32, i32, "items") if n else None,
+                                    n, gptr.data_ptr(), gnodes.data_ptr() if flat else None, len(groups), positions.data_ptr() if n else None,
+                                    cand.data_ptr() if n else None, n_cand.data_ptr(), _stream()), "recommend_filter")
+    return positions, cand, n_cand
+
+
+def recommend_topk_fused(tables, users: torch.Tensor, cand_items: torch.Tensor, k: int, exclude_ptr=None, exclude_items=None, slices=None,
+                         n_cand=None):
+    """Top-``k`` of ``cand_items`` for every row of ``users`` in one call, without a score matrix (``kgat_recommend_topk``).
+    ``tables``: the propagated layer tables [E0, ..., EL]; ``users`` / ``cand_items``: 1-D table rows, any integer dtype, candidates
+    unique; ``n_cand`` (device int32 [1], e.g. from ``recommend_filter``): only the first ``n_cand`` candidates count.
+    ``exclude_ptr`` int32 [>= max(users) + 2] / ``exclude_items`` int32: per user row the excluded item ids, ascending.  Scores
+    are bit-identical to ``sgemm_nt(gather_concat(...))``; order: score descending (``topk_rows`` key), then candidate index.
+    ``slices`` (1 .. 64, None = automatic) splits the candidates over CTAs; it does not change the result.
+    Returns ``(items int64 [U, k], scores fp32 [U, k], count int32 [U])`` padded with -1 / -inf after ``count``."""
+    k = int(k)
+    if not 1 <= k <= 128:
+        raise ValueError(f"k must be in [1, 128], got {k}")
+    if slices is not None and not 1 <= int(slices) <= 64:
+        raise ValueError(f"slices must be in [1, 64], got {slices}")
+    if (exclude_ptr is None) != (exclude_items is None):
+        raise ValueError("exclude_ptr and exclude_items go together")
+    dev = tables[0].device
+    rows = tables[0].shape[0]
+    users = _ids64(users, "users", dev)
+    cand_items = _ids64(cand_items, "cand_items", dev)
+    checks = [("user ids", users, rows), ("candidate ids", cand_items, rows)]
+    if exclude_ptr is not None:
+        if exclude_ptr.dim() != 1 or exclude_ptr.numel() < 2:
+            raise ValueError("exclude_ptr must be 1-D with one entry per user row plus one")
+        checks.append(("user ids (rows of exclude_ptr)", users, exclude_ptr.numel() - 1))
+    users32, cand32 = range_check(checks, dev)[:2] if users.numel() else (users.to(i32), cand_items.to(i32))
+    return launch_recommend_topk(tables, users32, cand32, k, exclude_ptr, exclude_items, slices, n_cand)
+
+
+def launch_recommend_topk(tables, users32: torch.Tensor, cand32: torch.Tensor, k: int, exclude_ptr=None, exclude_items=None, slices=None,
+                          n_cand=None):
+    """``recommend_topk_fused`` for int32 ids and arguments already known to be valid (no checks, no synchronisation)."""
+    lib = _lib.load()
+    dev = tables[0].device
+    t = _tables(tables)
+    U, n = users32.numel(), cand32.numel()
+    out_items = torch.empty(U, k, dtype=i64, device=dev)
+    out_scores = torch.empty(U, k, dtype=f32, device=dev)
+    out_count = torch.empty(U, dtype=i32, device=dev)
+    if U == 0:
+        return out_items, out_scores, out_count
+    s = 0 if slices is None else int(slices)
+    ws_bytes = int(lib.kgat_recommend_workspace_bytes(C.byref(t), U, n, k, s))
+    if ws_bytes < 0:
+        raise KgatLibraryError(f"recommend_topk: tables of width {sum(x.shape[1] for x in tables)} rejected (not multiples of 4, or too wide for shared memory at k = {k})")
+    ws = torch.empty(max(ws_bytes, 1), dtype=u8, device=dev)
+    check(lib.kgat_recommend_topk(
+        C.byref(t), _ptr(users32, i32, "users"), U, _ptr(cand32, i32, "cand_items") if n else None, n,
+        None if n_cand is None else _ptr(n_cand, i32, "n_cand"), k,
+        None if exclude_ptr is None else _ptr(exclude_ptr, i32, "exclude_ptr"), None if exclude_items is None else _ptr(exclude_items, i32, "exclude_items"),
+        s, out_items.data_ptr(), out_scores.data_ptr(), out_count.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "recommend_topk")
+    return out_items, out_scores, out_count
+
+
 # ----------------------------------------------------------------------------------------------
 # K11 Adam
 # ----------------------------------------------------------------------------------------------
