@@ -32,7 +32,7 @@ extern "C" {
 #define KGAT_ERR_UNSUPPORTED (-3)
 #define KGAT_ERR_WORKSPACE (-4)
 
-#define KGAT_ABI_VERSION 11
+#define KGAT_ABI_VERSION 12
 #define KGAT_MAX_LAYERS 8   /* embedding table + up to 7 propagation layers */
 #define KGAT_MAX_TENSORS 24 /* tensors per multi-tensor Adam launch */
 #define KGAT_MAX_PEERS 31   /* other ranks of a row-sharded propagation */
@@ -412,6 +412,30 @@ int64_t kgat_recommend_workspace_bytes(const kgat_tables_t* tables, int64_t n_us
 int kgat_recommend_topk(const kgat_tables_t* tables, const int32_t* users, int64_t n_users, const int32_t* cand_items, int64_t n_cand_max,
                         const int32_t* n_cand, int32_t k, const int32_t* exclude_ptr, const int32_t* exclude_items, int32_t slices,
                         int64_t* out_items, float* out_scores, int32_t* out_count, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------- */
+/* Exact full ranking of held-out targets (the full-ranking metrics: rank, MRR, AUC, any k)      */
+/* ------------------------------------------------------------------------------------------- */
+/* For every users[b] (int32 table row) and each of its targets p = target_items[target_ptr[u] .. target_ptr[u+1]) (ascending,
+ * table rows), the exact number of eligible candidates that outrank p.  Candidates: cand_items[0 .. n_cand) (int32 table rows,
+ * unique); the position of an item is given by pos_map[item] (int32 [n_pos], -1 when not a candidate) or, when pos_map is
+ * NULL, by the item itself (then cand_items[c] must be c).  exclude_ptr / exclude_items (nullable): CSR over table rows of
+ * users, items ascending; an excluded item is not eligible.  Score s(b, c) as in kgat_recommend_topk; key K(b, c) =
+ * (topk_rows key of s << 32) | (0xFFFFFFFF - position of c), the order of kgat_recommend_topk.  Outputs, row b at
+ * out_ptr[b] .. out_ptr[b+1] (int64 [n_users + 1], out_ptr[b+1] - out_ptr[b] = number of targets of users[b],
+ * out_ptr[n_users] = n_targets):
+ *   out_items    int64 [n_targets]  the targets, ascending
+ *   out_scores   fp32  [n_targets]  s(b, p), bit-identical to kgat_gather_concat + kgat_sgemm_nt
+ *   out_rank     int64 [n_targets]  #{eligible c : K(b, c) > K(b, p)}, or -1 when p is not eligible
+ *   out_eligible int64 [n_users]    number of eligible candidates of users[b]
+ * slices in [0, 64] = candidate slices per 64-user tile (0 = the rule of kgat_recommend_topk; the result does not depend on
+ * it).  Three launches, no host synchronisation; workspace from kgat_rank_workspace_bytes (-1 for invalid arguments or a row
+ * too wide for shared memory, when kgat_rank_targets returns KGAT_ERR_UNSUPPORTED). */
+int64_t kgat_rank_workspace_bytes(const kgat_tables_t* tables, int64_t n_users, int64_t n_targets);
+int kgat_rank_targets(const kgat_tables_t* tables, const int32_t* users, int64_t n_users, const int32_t* cand_items, int64_t n_cand,
+                      const int32_t* pos_map, int64_t n_pos, const int32_t* target_ptr, const int32_t* target_items, const int64_t* out_ptr,
+                      int64_t n_targets, const int32_t* exclude_ptr, const int32_t* exclude_items, int32_t slices, int64_t* out_items,
+                      float* out_scores, int64_t* out_rank, int64_t* out_eligible, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* K11: Adam                               reference model.py:393-419 (torch.optim.Adam)       */

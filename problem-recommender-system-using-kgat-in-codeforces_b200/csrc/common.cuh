@@ -123,6 +123,91 @@ inline bool tables_from(const kgat_tables_t* t, ConcatTables* T) {
     return true;
 }
 
+inline int padded_width(const ConcatTables& T) { return ((T.qoff[T.n] * 4 + 15) / 16) * 16; }
+
+// float4 of concatenated columns [4 q, 4 q + 4) of table row `id` (zeros past the width)
+__device__ __forceinline__ float4 concat_quad(const ConcatTables& T, int64_t id, int q) {
+    int t = 0;
+    while (t < T.n && q >= T.qoff[t + 1]) ++t;
+    if (t == T.n) return make_float4(0.f, 0.f, 0.f, 0.f);
+    return ldg4(T.p[t] + id * T.ld[t] + (q - T.qoff[t]) * 4);
+}
+
+// ------------------------------------------------------------------------------------------
+// 64-user x 64-candidate score tiles of the fused scoring kernels (recommend.cu, rank.cu): 256 threads, thread (tx, ty) =
+// (tid % 16, tid / 16) owns users ty * 4 + i and candidates tx * 4 + j of a tile.  The arithmetic is sgemm_nt_kernel's:
+// a sequential fmaf chain from +0 over the concatenated columns in ascending order, zero-padded to a multiple of 16.
+// ------------------------------------------------------------------------------------------
+constexpr int kTileThreads = 256;
+constexpr int kTileUsers = 64;
+constexpr int kTileItems = 64;
+constexpr int kTilePad = 68;       // shared row stride (floats) of the transposed tiles, as in sgemm_nt_kernel
+constexpr int kTileMaxSlices = 64;
+
+// shared floats of the user tile [width_pad][kTilePad] and the candidate slab [16][kTilePad]
+inline size_t tile_smem_floats(int width_pad) { return (size_t)(width_pad + 16) * kTilePad; }
+
+// Us[c][r] = column c of users[u0 + r]'s concatenated row (zero rows past n_users).  The caller synchronises afterwards.
+__device__ __forceinline__ void stage_user_tile(const ConcatTables& T, const int32_t* __restrict__ users, int n_users, int u0, int width_pad,
+                                                float* Us) {
+    const int nq = width_pad / 4;
+    for (int e = threadIdx.x; e < kTileUsers * nq; e += kTileThreads) {
+        const int r = e % kTileUsers, q = e / kTileUsers;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (u0 + r < n_users) v = concat_quad(T, users[u0 + r], q);
+        Us[(4 * q + 0) * kTilePad + r] = v.x;
+        Us[(4 * q + 1) * kTilePad + r] = v.y;
+        Us[(4 * q + 2) * kTilePad + r] = v.z;
+        Us[(4 * q + 3) * kTilePad + r] = v.w;
+    }
+}
+
+// acc[i][j] = score of staged user ty * 4 + i and candidate c0 + tx * 4 + j (candidates from c_end on score 0).  Every thread
+// of the CTA calls it; it synchronises before each write of the slab Bs, so the caller may read acc without a barrier.
+__device__ __forceinline__ void score_tile(const ConcatTables& T, const int32_t* __restrict__ cand, int c0, int c_end, int width_pad, const float* Us,
+                                           float* Bs, float (&acc)[4][4]) {
+    const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
+    const int lr = tid / 4, lk = (tid % 4) * 4;  // slab load mapping: 64 candidates x 16 columns, one float4 per thread
+    const int my_c = c0 + lr;
+    const int64_t my_id = my_c < c_end ? cand[my_c] : -1;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+    for (int k0 = 0; k0 < width_pad; k0 += 16) {
+        const float4 b = my_id >= 0 ? concat_quad(T, my_id, (k0 + lk) / 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+        __syncthreads();
+        Bs[(lk + 0) * kTilePad + lr] = b.x;
+        Bs[(lk + 1) * kTilePad + lr] = b.y;
+        Bs[(lk + 2) * kTilePad + lr] = b.z;
+        Bs[(lk + 3) * kTilePad + lr] = b.w;
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < 16; ++kk) {
+            const float4 av = *reinterpret_cast<const float4*>(&Us[(k0 + kk) * kTilePad + ty * 4]);
+            const float4 bv = *reinterpret_cast<const float4*>(&Bs[kk * kTilePad + tx * 4]);
+            const float ar[4] = {av.x, av.y, av.z, av.w}, br[4] = {bv.x, bv.y, bv.z, bv.w};
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(ar[i], br[j], acc[i][j]);
+        }
+    }
+}
+
+// candidate slices per 64-user tile: enough CTAs for two waves over the SMs while the users alone do not give them (per_sm =
+// resident CTAs per SM of the kernel), at least one 64-candidate tile per slice; `requested` > 0 is taken as is
+inline int pick_slices(int64_t n_users, int64_t n_cand_max, int per_sm, int requested) {
+    if (requested > 0) return requested;
+    const int64_t tiles = (n_users + kTileUsers - 1) / kTileUsers;
+    const int64_t want = 2LL * sm_count() * per_sm;
+    int64_t s = tiles > 0 ? (want + tiles - 1) / tiles : 1;
+    const int64_t by_items = (n_cand_max + kTileItems - 1) / kTileItems;
+    if (s > by_items) s = by_items;
+    if (s > kTileMaxSlices) s = kTileMaxSlices;
+    return (int)(s < 1 ? 1 : s);
+}
+
 // log(sigmoid(x)) as ATen computes it: min(x,0) - log1p(exp(-|x|))
 __device__ __forceinline__ float log_sigmoid(float x) { return fminf(x, 0.f) - log1pf(expf(-fabsf(x))); }
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }

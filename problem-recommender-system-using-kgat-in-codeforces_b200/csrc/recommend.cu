@@ -18,12 +18,11 @@
 namespace kgat {
 namespace {
 
-constexpr int kRecThreads = 256;
-constexpr int kRecUsers = 64;     // users per CTA
-constexpr int kRecItems = 64;     // candidates per tile
-constexpr int kRecMaxK = 128;     // = kTopkMax of topk_rows
-constexpr int kRecMaxSlices = 64;
-constexpr int kRecPad = 68;       // shared row stride (floats) of the transposed tiles, as in sgemm_nt_kernel
+constexpr int kRecThreads = kTileThreads;
+constexpr int kRecUsers = kTileUsers;  // users per CTA
+constexpr int kRecItems = kTileItems;  // candidates per tile
+constexpr int kRecMaxK = 128;          // = kTopkMax of topk_rows
+constexpr int kRecMaxSlices = kTileMaxSlices;
 
 struct Entry {
     float s;
@@ -57,23 +56,8 @@ inline int64_t workspace_bytes(int64_t n_users, int slices, int k) {
     return align256(n_users * slices * k * (int64_t)sizeof(Entry)) + align256(n_users * slices * 4);
 }
 
-inline int padded_width(const ConcatTables& T) { return ((T.qoff[T.n] * 4 + 15) / 16) * 16; }
-
 inline size_t score_smem_bytes(int width_pad, int k) {
-    return sizeof(float) * (size_t)(width_pad + 16) * kRecPad + sizeof(Entry) * (size_t)kRecUsers * (k + kRecItems) + 2 * sizeof(int) * kRecUsers;
-}
-
-// slices per 64-user tile: enough CTAs for two waves over the SMs while the users alone do not give them (per_sm = resident
-// score CTAs per SM), at least one 64-candidate tile per slice
-int pick_slices(int64_t n_users, int64_t n_cand_max, int per_sm, int requested) {
-    if (requested > 0) return requested;
-    const int64_t tiles = (n_users + kRecUsers - 1) / kRecUsers;
-    const int64_t want = 2LL * sm_count() * per_sm;
-    int64_t s = tiles > 0 ? (want + tiles - 1) / tiles : 1;
-    const int64_t by_items = (n_cand_max + kRecItems - 1) / kRecItems;
-    if (s > by_items) s = by_items;
-    if (s > kRecMaxSlices) s = kRecMaxSlices;
-    return (int)(s < 1 ? 1 : s);
+    return sizeof(float) * tile_smem_floats(width_pad) + sizeof(Entry) * (size_t)kRecUsers * (k + kRecItems) + 2 * sizeof(int) * kRecUsers;
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -153,20 +137,12 @@ struct ScoreArgs {
     int32_t* ws_len;            // [n_users][slices]
 };
 
-// float4 of concatenated columns [4 q, 4 q + 4) of table row `id` (zeros past the width)
-__device__ __forceinline__ float4 concat_quad(const ConcatTables& T, int64_t id, int q) {
-    int t = 0;
-    while (t < T.n && q >= T.qoff[t + 1]) ++t;
-    if (t == T.n) return make_float4(0.f, 0.f, 0.f, 0.f);
-    return ldg4(T.p[t] + id * T.ld[t] + (q - T.qoff[t]) * 4);
-}
-
 __global__ void __launch_bounds__(kRecThreads) recommend_score_kernel(ScoreArgs a) {
     extern __shared__ float4 smem_f4[];
-    float* Us = reinterpret_cast<float*>(smem_f4);            // [width_pad][kRecPad]: the tile's users, transposed
-    float* Bs = Us + (size_t)a.width_pad * kRecPad;           // [16][kRecPad]: one 16-column slab of a candidate tile
-    Entry* top = reinterpret_cast<Entry*>(Bs + 16 * kRecPad); // [kRecUsers][k], sorted best-first
-    Entry* pend = top + kRecUsers * a.k;                      // [kRecUsers][kRecItems], unordered
+    float* Us = reinterpret_cast<float*>(smem_f4);              // [width_pad][kTilePad]: the tile's users, transposed
+    float* Bs = Us + (size_t)a.width_pad * kTilePad;            // [16][kTilePad]: one 16-column slab of a candidate tile
+    Entry* top = reinterpret_cast<Entry*>(Bs + 16 * kTilePad);  // [kRecUsers][k], sorted best-first
+    Entry* pend = top + kRecUsers * a.k;                        // [kRecUsers][kRecItems], unordered
     int* n_top = reinterpret_cast<int*>(pend + kRecUsers * kRecItems);
     int* n_pend = n_top + kRecUsers;
 
@@ -178,16 +154,7 @@ __global__ void __launch_bounds__(kRecThreads) recommend_score_kernel(ScoreArgs 
     const int c_begin = (int)((int64_t)n_cand * slice / a.slices), c_end = (int)((int64_t)n_cand * (slice + 1) / a.slices);
 
     // stage the users' concatenated rows (zero rows past n_users, zero columns past the width)
-    const int nq = a.width_pad / 4;
-    for (int e = tid; e < kRecUsers * nq; e += kRecThreads) {
-        const int r = e % kRecUsers, q = e / kRecUsers;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (u0 + r < a.n_users) v = concat_quad(a.T, a.users[u0 + r], q);
-        Us[(4 * q + 0) * kRecPad + r] = v.x;
-        Us[(4 * q + 1) * kRecPad + r] = v.y;
-        Us[(4 * q + 2) * kRecPad + r] = v.z;
-        Us[(4 * q + 3) * kRecPad + r] = v.w;
-    }
+    stage_user_tile(a.T, a.users, a.n_users, u0, a.width_pad, Us);
     if (tid < kRecUsers) { n_top[tid] = 0; n_pend[tid] = 0; }
 
     // per-thread exclusion ranges of its 4 users
@@ -204,30 +171,9 @@ __global__ void __launch_bounds__(kRecThreads) recommend_score_kernel(ScoreArgs 
     }
     __syncthreads();
 
-    const int lr = tid / 4, lk = (tid % 4) * 4;  // slab load mapping: 64 candidates x 16 columns, one float4 per thread
     for (int c0 = c_begin; c0 < c_end; c0 += kRecItems) {
-        const int my_c = c0 + lr;
-        const int64_t my_id = my_c < c_end ? a.cand[my_c] : -1;
-        float acc[4][4] = {};
-        for (int k0 = 0; k0 < a.width_pad; k0 += 16) {
-            const float4 b = my_id >= 0 ? concat_quad(a.T, my_id, (k0 + lk) / 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-            __syncthreads();
-            Bs[(lk + 0) * kRecPad + lr] = b.x;
-            Bs[(lk + 1) * kRecPad + lr] = b.y;
-            Bs[(lk + 2) * kRecPad + lr] = b.z;
-            Bs[(lk + 3) * kRecPad + lr] = b.w;
-            __syncthreads();
-#pragma unroll
-            for (int kk = 0; kk < 16; ++kk) {
-                const float4 av = *reinterpret_cast<const float4*>(&Us[(k0 + kk) * kRecPad + ty * 4]);
-                const float4 bv = *reinterpret_cast<const float4*>(&Bs[kk * kRecPad + tx * 4]);
-                const float ar[4] = {av.x, av.y, av.z, av.w}, br[4] = {bv.x, bv.y, bv.z, bv.w};
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(ar[i], br[j], acc[i][j]);
-            }
-        }
+        float acc[4][4];
+        score_tile(a.T, a.cand, c0, c_end, a.width_pad, Us, Bs, acc);
         // admission: beats the user's k-th entry (or the list is not full) and is not excluded
         bool any = false;
 #pragma unroll

@@ -113,3 +113,80 @@ def evaluate(model, train: InteractionCSR, test: InteractionCSR, k_list=(20, 40,
         n_done += ub.shape[0]
     out = {k: {m: v / max(n_done, 1) for m, v in d.items()} for k, d in sums.items()}
     return out, (torch.cat(tops) if tops else torch.zeros(0, kmax, dtype=torch.int64, device=dev))
+
+
+def metrics_from_ranks(ranks, n_test: np.ndarray, k_list) -> torch.Tensor:
+    """Mean ranking metrics of the rows of ``ranks`` (a ``model.TargetRanks``, or anything with its fields) as one fp64 tensor:
+    for each k of ``k_list`` precision, recall, ndcg and hit, then mrr, auc and mean_rank (see ``rank_metrics``).  ``n_test``
+    (host array): the denominator ``T_u`` of each row.  Per-row terms in fp64 (integer counts exact), each row summed in target order and the
+    rows summed in a fixed order, so the result is deterministic; works on CPU or CUDA tensors alike."""
+    dev = ranks.rank.device
+    U = ranks.ptr.numel() - 1
+    rk = ranks.rank
+    seg = torch.repeat_interleave(torch.arange(U, device=dev), ranks.ptr.diff(), output_size=rk.numel())
+    valid = rk >= 0
+    max_t = int(min(max(k_list), max(int(n_test.max()) if U else 0, 1)))  # the ideal DCG needs min(k, T_u) <= max_t terms
+    n_test = torch.from_numpy(np.asarray(n_test, dtype=np.float64)).to(dev)
+
+    def per_row(x):  # integer sum per row
+        return torch.zeros(U, dtype=torch.int64, device=dev).index_add_(0, seg, x.to(torch.int64)).to(torch.float64)
+
+    def mean(x, mask=None):
+        if mask is None:
+            return x.sum() / max(U, 1)
+        return torch.where(mask, x, 0.0).sum() / mask.sum().clamp(min=1)
+
+    cum_ideal = torch.from_numpy(np.cumsum(1.0 / np.log2(np.arange(2, max_t + 2, dtype=np.float64)))).to(dev)
+    gain = torch.where(valid, 1.0 / torch.log2(rk.clamp(min=0).to(torch.float64) + 2.0), 0.0)
+    out = []
+    for k in k_list:
+        in_k = valid & (rk < k)
+        h = per_row(in_k)
+        dcg = torch.segment_reduce(torch.where(in_k, gain, 0.0), "sum", offsets=ranks.ptr, unsafe=True)
+        n_ideal = n_test.clamp(max=k).to(torch.int64)
+        idcg = torch.where(n_ideal > 0, cum_ideal[(n_ideal - 1).clamp(min=0, max=max_t - 1)], float("inf"))
+        out += [mean(h / k), mean(h / n_test), mean(dcg / idcg), mean((h > 0).to(torch.float64))]
+    P = per_row(valid)
+    S = per_row(torch.where(valid, rk, 0))
+    big = torch.iinfo(torch.int64).max
+    best = torch.full((U,), big, dtype=torch.int64, device=dev).scatter_reduce_(0, seg, torch.where(valid, rk, big), "amin")
+    mrr = torch.where(P > 0, 1.0 / (1.0 + best.clamp(max=2**53).to(torch.float64)), 0.0)
+    N = ranks.eligible.to(torch.float64) - P
+    auc = 1.0 - (S - P * (P - 1) / 2) / (P * N)
+    out += [mean(mrr), mean(auc, (P > 0) & (N > 0)), mean(S / P, P > 0)]
+    return torch.stack(out)
+
+
+@torch.no_grad()
+def rank_metrics(model, train: InteractionCSR, test: InteractionCSR, k_list=(20, 40, 60, 80, 100), users=None) -> dict:
+    """Full-ranking metrics of ``users`` (default: every user with at least one test item, as ``evaluate``), from the exact rank
+    of each test item among all problems not in the user's training positives (``model.rank(users, train.item_num, test,
+    exclude=train)``); no score matrix.  With ``T_u`` = the user's number of test items (``evaluate``'s denominator) and
+    ``h_k`` = the test items of rank < k, per user:
+
+        precision@k = h_k / k                  recall@k = h_k / T_u (NaN when T_u = 0, as the reference)
+        ndcg@k      = sum_{rank < k} 1 / log2(rank + 2)  /  sum_{i < min(k, T_u)} 1 / log2(i + 2)
+        hit@k       = [h_k > 0]                mrr = 1 / (1 + lowest rank), 0 when no test item is eligible
+        mean_rank   = the mean rank of the user's eligible test items
+        auc         = 1 - sum_i (r_(i) - i) / (P' N'), r_(0) < r_(1) < ... the eligible test items' ranks, P' their number,
+                      N' = eligible problems - P': the fraction of (test item, other eligible problem) pairs ordered correctly
+
+    A test item that is also a training positive is not eligible: it counts in ``T_u`` but has no rank.  Users without an
+    eligible test item, or without any other eligible problem, have no AUC and no mean rank, and are left out of those two
+    means; every other metric is the mean over all ``users``.  ``k`` may be any positive int.  Exactly the top-k that
+    ``evaluate`` sees for k <= 128 when the user has at least k eligible problems (``evaluate`` then has no masked entry in its
+    top-k).  Per-user terms are computed on the device in fp64 and reduced in a fixed order; the result is read back once.
+
+    Returns ``{k: {"precision", "recall", "ndcg", "hit"} for k in k_list, "mrr": float, "auc": float, "mean_rank": float}``."""
+    k_list = [int(k) for k in k_list]
+    if not k_list or min(k_list) < 1:
+        raise ValueError(f"k_list must hold positive ints, got {k_list}")
+    model.eval()
+    if users is None:
+        users = np.nonzero(np.diff(test.ptr_host) > 0)[0]
+    users = torch.as_tensor(np.asarray(users, dtype=np.int64))
+    ranks = model.rank(users, train.item_num, test, exclude=train)
+    vals = metrics_from_ranks(ranks, np.diff(test.ptr_host)[users.numpy()], k_list).tolist()
+    out: dict = {k: dict(zip(("precision", "recall", "ndcg", "hit"), vals[4 * j : 4 * j + 4])) for j, k in enumerate(k_list)}
+    out.update(zip(("mrr", "auc", "mean_rank"), vals[4 * len(k_list) :]))
+    return out

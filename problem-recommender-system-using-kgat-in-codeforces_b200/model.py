@@ -76,6 +76,18 @@ class Recommendation:
     count: torch.Tensor  # int32 [U]: min(k, number of eligible problems)
 
 
+@dataclass
+class TargetRanks:
+    """Result of ``KGAT.rank`` for U users and M targets in all: row ``b`` is ``ptr[b] .. ptr[b+1]``, the targets of ``user_ids[b]``
+    in ascending id."""
+
+    ptr: torch.Tensor  # int64 [U+1]
+    items: torch.Tensor  # int64 [M]: problem ids
+    scores: torch.Tensor  # fp32 [M]: the PREDICT scores of those problems
+    rank: torch.Tensor  # int64 [M]: eligible problems ranked before the target (0 = first), -1 when the target is not eligible
+    eligible: torch.Tensor  # int64 [U]: number of eligible problems of the user
+
+
 class KGATMode(IntEnum):
     TRAIN_CF = 0
     TRAIN_KG = 1
@@ -620,6 +632,25 @@ class KGAT(nn.Module):
         if not 1 <= k <= 128:
             raise ValueError(f"k must be in [1, 128], got {k}")
         dev = self._device()
+        users, cand = self._users_and_items(user_ids, items, exclude)
+        if require is not None:
+            require = ops.require_groups(require, self._entity_num)
+        # ranges and duplicates in one read-back: the only host synchronisation of the call
+        dup = ops.duplicate_count(cand)
+        users32, cand32 = ops.range_check([("user ids", users, self._user_num), ("item ids", cand, self._entity_num)], dev,
+                                          flags=[("items holds duplicate ids", dup)])
+        tables = self._tables()
+        n_cand = None
+        if require is not None:
+            _, cand32, n_cand = ops.launch_recommend_filter(self._graph(), cand32, require, self._user_num)
+        ex_ptr, ex_items = (exclude.ptr_dev.to(dev), exclude.items.to(dev)) if exclude is not None else (None, None)
+        out_items, scores, count = ops.launch_recommend_topk(tables, users32, cand32, k, ex_ptr, ex_items, n_cand=n_cand)
+        return Recommendation(items=out_items, scores=scores, count=count)
+
+    def _users_and_items(self, user_ids, items, exclude):
+        """``user_ids`` / ``items`` of ``recommend`` and ``rank`` as int64 on the device (ranges are checked by the caller's
+        read-back); ValueError for a malformed argument or an ``exclude`` over another number of users."""
+        dev = self._device()
         users = torch.as_tensor(user_ids)
         if users.dim() != 1 or users.dtype not in (torch.int32, torch.int64):
             raise ValueError(f"user_ids must be a 1-D int32 / int64 tensor, got {users.dtype} of shape {tuple(users.shape)}")
@@ -635,19 +666,45 @@ class KGAT(nn.Module):
             cand = cand.to(device=dev, dtype=torch.int64)
         if exclude is not None and exclude.user_num != self._user_num:
             raise ValueError(f"exclude covers {exclude.user_num} users, the model has {self._user_num}")
-        if require is not None:
-            require = ops.require_groups(require, self._entity_num)
-        # ranges and duplicates in one read-back: the only host synchronisation of the call
-        dup = (torch.sort(cand).values.diff() == 0).sum() if cand.numel() > 1 else torch.zeros((), dtype=torch.int64, device=dev)
-        users32, cand32 = ops.range_check([("user ids", users, self._user_num), ("item ids", cand, self._entity_num)], dev,
-                                          flags=[("items holds duplicate ids", dup)])
+        return users, cand
+
+    @torch.no_grad()
+    def rank(self, user_ids, items, targets, exclude=None) -> "TargetRanks":
+        """The exact rank of every held-out problem of every listed user among ``items``, in one call, without a score matrix.
+
+        ``user_ids``, ``items`` and ``exclude`` are those of ``recommend`` (ints / tensors, repeats of users allowed, ``items``'
+        order breaks score ties).  ``targets``: a ``metrics.InteractionCSR`` over the same ``user_num`` of the problems to rank,
+        e.g. the test split; row ``b`` of the result holds ``targets[user_ids[b]]`` in ascending id.
+
+        Score ``s(u, c)``: the fp32 ``model(u, c, mode=PREDICT)`` value (the sequential ``fmaf`` chain over ``E0|...|EL``,
+        zero-padded to 16 columns; quirk Q4: row ``c``).  Key ``K(u, c) = (float_key(s) << 32) | (0xFFFFFFFF - pos(c))``, ``pos``
+        the position in ``items``: ``recommend``'s order.  A problem is eligible for ``u`` when it is in ``items`` and not in
+        ``exclude[u]``.  For an eligible target ``p``::
+
+            rank(u, p) = #{c eligible for u : K(u, c) > K(u, p)}
+
+        so ``rank < k <= 128`` means ``recommend(u, items, k, exclude).items[b, rank] == p``.  A target that is not eligible gets
+        rank -1 (its score is still given).  ``eligible[b]`` counts the eligible problems of ``u``.  Only integers are counted, so
+        the result does not depend on how the GPU splits the work.
+
+        ValueError for every argument ``recommend`` rejects, for ``targets`` over another number of users, and for ``targets``
+        whose item range exceeds ``entity_num``.  Uses the cached propagation after settling deferred KG rows, and honours train /
+        eval mode as PREDICT does: call it in ``eval()``.  One host synchronisation (the range-check read-back)."""
+        dev = self._device()
+        users, cand = self._users_and_items(user_ids, items, exclude)
+        if targets.user_num != self._user_num:
+            raise ValueError(f"targets cover {targets.user_num} users, the model has {self._user_num}")
+        if targets.item_num > self._entity_num:
+            raise ValueError(f"targets hold problem ids up to {targets.item_num - 1}, the model has {self._entity_num} entities")
+        t_ptr, t_items = targets.ptr_dev.to(dev), targets.items.to(dev)
+        out_ptr = ops.target_rows(t_ptr, users)
+        users32, cand32, n_targets = ops.range_check([("user ids", users, self._user_num), ("item ids", cand, self._entity_num)], dev,
+                                                     flags=[("items holds duplicate ids", ops.duplicate_count(cand))], values=[out_ptr[-1]])
         tables = self._tables()
-        n_cand = None
-        if require is not None:
-            _, cand32, n_cand = ops.launch_recommend_filter(self._graph(), cand32, require, self._user_num)
         ex_ptr, ex_items = (exclude.ptr_dev.to(dev), exclude.items.to(dev)) if exclude is not None else (None, None)
-        out_items, scores, count = ops.launch_recommend_topk(tables, users32, cand32, k, ex_ptr, ex_items, n_cand=n_cand)
-        return Recommendation(items=out_items, scores=scores, count=count)
+        ptr, t, scores, rank, eligible = ops.launch_rank(tables, users32, cand32, t_ptr, t_items, out_ptr, n_targets, ex_ptr, ex_items,
+                                                         arange=isinstance(items, int), n_pos=self._entity_num)
+        return TargetRanks(ptr=ptr, items=t, scores=scores, rank=rank, eligible=eligible)
 
     @torch.no_grad()
     def explain(self, user_ids, item_ids, k: int = 10, max_hops: int | None = None) -> "PathExplanation":

@@ -723,10 +723,11 @@ def _ids64(ids: torch.Tensor, name: str, dev) -> torch.Tensor:
     return ids.to(device=dev, dtype=i64).contiguous()
 
 
-def range_check(checks, dev, flags=()) -> list:
-    """checks: (name, int64 ids on dev, bound >= 1); flags: (message, device integer scalar that is nonzero on failure).
-    Converts every id list to int32 and reads the out-of-range counts and the flags back in one synchronisation, before any
-    kernel indexes with the ids; ValueError for the first check or flag that fails.  Returns the int32 id lists."""
+def range_check(checks, dev, flags=(), values=()) -> list:
+    """checks: (name, int64 ids on dev, bound >= 1); flags: (message, device integer scalar that is nonzero on failure);
+    values: device integer scalars the caller needs on the host.  Converts every id list to int32 and reads the out-of-range
+    counts, the flags and the values back in one synchronisation, before any kernel indexes with the ids; ValueError for the
+    first check or flag that fails.  Returns the int32 id lists, followed by the values as ints."""
     lib = _lib.load()
     bad = torch.zeros(len(checks) + len(flags), dtype=i32, device=dev)
     outs = []
@@ -737,14 +738,17 @@ def range_check(checks, dev, flags=()) -> list:
         outs.append(out)
     for j, (_, flag) in enumerate(flags):
         bad[len(checks) + j] = flag
-    got = bad.tolist()
+    if values:
+        got = torch.cat([bad.to(i64), torch.stack([torch.as_tensor(v, device=dev).to(i64).reshape(()) for v in values])]).tolist()
+    else:
+        got = bad.tolist()
     for (name, _, bound), n_bad in zip(checks, got):
         if n_bad:
             raise ValueError(f"{n_bad} {name} outside [0, {bound})")
     for (msg, _), n_bad in zip(flags, got[len(checks) :]):
         if n_bad:
             raise ValueError(msg)
-    return outs
+    return outs + got[len(checks) + len(flags) :]
 
 
 def require_groups(groups, n_ent: int):
@@ -841,6 +845,96 @@ def launch_recommend_topk(tables, users32: torch.Tensor, cand32: torch.Tensor, k
         None if exclude_ptr is None else _ptr(exclude_ptr, i32, "exclude_ptr"), None if exclude_items is None else _ptr(exclude_items, i32, "exclude_items"),
         s, out_items.data_ptr(), out_scores.data_ptr(), out_count.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "recommend_topk")
     return out_items, out_scores, out_count
+
+
+def duplicate_count(ids: torch.Tensor) -> torch.Tensor:
+    """Device scalar: the number of repeated entries of the 1-D ``ids`` (0 when they are unique)."""
+    if ids.numel() < 2:
+        return torch.zeros((), dtype=i64, device=ids.device)
+    return (torch.sort(ids).values.diff() == 0).sum()
+
+
+def target_rows(target_ptr: torch.Tensor, users: torch.Tensor) -> torch.Tensor:
+    """Row pointer (int64 [U + 1], on the device) of the targets of ``users`` (int64) under the CSR pointer ``target_ptr``.  Ids
+    outside the pointer's rows are clamped, so this is safe before the range check; the pointer is meaningful after it."""
+    cnt = (target_ptr[1:] - target_ptr[:-1]).to(i64)
+    out = torch.zeros(users.numel() + 1, dtype=i64, device=users.device)
+    if users.numel() and cnt.numel():
+        torch.cumsum(cnt[users.clamp(0, cnt.numel() - 1)], 0, out=out[1:])
+    return out
+
+
+def rank_targets(tables, users: torch.Tensor, cand_items, target_ptr: torch.Tensor, target_items: torch.Tensor, exclude_ptr=None,
+                 exclude_items=None, slices=None):
+    """Exact rank of every target of every row of ``users`` among ``cand_items`` in one call, without a score matrix
+    (``kgat_rank_targets``).  ``tables``: the propagated layer tables [E0, ..., EL]; ``users``: 1-D table rows, any integer dtype,
+    repeats allowed; ``cand_items``: an int ``n`` (= ``arange(n)``) or 1-D unique table rows, whose order breaks score ties;
+    ``target_ptr`` int32 [>= max(users) + 2] / ``target_items`` int32: per user row the targets, ascending;
+    ``exclude_ptr`` / ``exclude_items``: per user row the excluded item ids, ascending (an excluded item is not eligible).
+    ``rank`` = the number of eligible candidates whose (score, position) key beats the target's, the order of
+    ``recommend_topk_fused``; -1 when the target is not an eligible candidate.  ``slices`` (1 .. 64, None = automatic) does not
+    change the result.  Returns ``(ptr int64 [U+1], items int64 [M], scores fp32 [M], rank int64 [M], eligible int64 [U])``."""
+    if slices is not None and not 1 <= int(slices) <= 64:
+        raise ValueError(f"slices must be in [1, 64], got {slices}")
+    if (exclude_ptr is None) != (exclude_items is None):
+        raise ValueError("exclude_ptr and exclude_items go together")
+    if target_ptr.dim() != 1 or target_ptr.numel() < 2:
+        raise ValueError("target_ptr must be 1-D with one entry per user row plus one")
+    dev = tables[0].device
+    rows = tables[0].shape[0]
+    users = _ids64(users, "users", dev)
+    arange = isinstance(cand_items, int)
+    if arange and not 0 <= cand_items <= rows:
+        raise ValueError(f"cand_items = {cand_items} must lie in [0, {rows}]")
+    cand = torch.arange(cand_items, device=dev) if arange else _ids64(cand_items, "cand_items", dev)
+    target_ptr, target_items = target_ptr.to(dev), target_items.to(dev)
+    checks = [("user ids", users, rows), ("candidate ids", cand, rows), ("user ids (rows of target_ptr)", users, target_ptr.numel() - 1)]
+    if exclude_ptr is not None:
+        if exclude_ptr.dim() != 1 or exclude_ptr.numel() < 2:
+            raise ValueError("exclude_ptr must be 1-D with one entry per user row plus one")
+        checks.append(("user ids (rows of exclude_ptr)", users, exclude_ptr.numel() - 1))
+    bad_targets = ((target_items < 0) | (target_items >= rows)).sum()
+    out_ptr = target_rows(target_ptr, users)
+    got = range_check(checks, dev, flags=[("cand_items holds duplicate ids", duplicate_count(cand)), (f"target ids outside [0, {rows})", bad_targets)],
+                      values=[out_ptr[-1]])
+    return launch_rank(tables, got[0], got[1], target_ptr, target_items, out_ptr, got[-1], exclude_ptr, exclude_items, slices, arange=arange,
+                       n_pos=rows)
+
+
+def launch_rank(tables, users32: torch.Tensor, cand32: torch.Tensor, target_ptr, target_items, out_ptr, n_targets: int, exclude_ptr=None,
+                exclude_items=None, slices=None, arange: bool = False, n_pos: int = 0):
+    """``rank_targets`` for int32 ids and arguments already known to be valid (no checks, no synchronisation).  ``out_ptr``
+    from ``target_rows`` with ``n_targets = out_ptr[-1]``; ``arange``: ``cand32`` is ``0 .. n - 1``, positions are the ids;
+    otherwise an int32 [n_pos] position map is built (every candidate id below ``n_pos``)."""
+    lib = _lib.load()
+    dev = tables[0].device
+    t = _tables(tables)
+    U, n, M = users32.numel(), cand32.numel(), int(n_targets)
+    items = torch.empty(M, dtype=i64, device=dev)
+    scores = torch.empty(M, dtype=f32, device=dev)
+    rank = torch.empty(M, dtype=i64, device=dev)
+    eligible = torch.empty(U, dtype=i64, device=dev)
+    if U == 0:
+        return out_ptr, items, scores, rank, eligible
+    if exclude_items is not None and exclude_items.numel() == 0:
+        exclude_ptr = exclude_items = None  # nothing is excluded
+    pos_map = None
+    if not arange:
+        pos_map = torch.full((max(int(n_pos), 1),), -1, dtype=i32, device=dev)
+        pos_map[cand32.long()] = torch.arange(n, dtype=i32, device=dev)
+    s = 0 if slices is None else int(slices)
+    ws_bytes = int(lib.kgat_rank_workspace_bytes(C.byref(t), U, M))
+    if ws_bytes < 0:
+        raise KgatLibraryError(f"rank_targets: tables of width {sum(x.shape[1] for x in tables)} rejected (not multiples of 4, or too wide for shared memory)")
+    ws = torch.empty(max(ws_bytes, 1), dtype=u8, device=dev)
+    check(lib.kgat_rank_targets(
+        C.byref(t), _ptr(users32, i32, "users"), U, _ptr(cand32, i32, "cand_items") if n else None, n,
+        None if pos_map is None else pos_map.data_ptr(), 0 if pos_map is None else pos_map.numel(), _ptr(target_ptr, i32, "target_ptr"),
+        _ptr(target_items, i32, "target_items") if M else None, _ptr(out_ptr, i64, "out_ptr"), M,
+        None if exclude_ptr is None else _ptr(exclude_ptr, i32, "exclude_ptr"), None if exclude_items is None else _ptr(exclude_items, i32, "exclude_items"),
+        s, items.data_ptr() if M else None, scores.data_ptr() if M else None, rank.data_ptr() if M else None, eligible.data_ptr(), ws.data_ptr(),
+        ws_bytes, _stream()), "rank_targets")
+    return out_ptr, items, scores, rank, eligible
 
 
 # ----------------------------------------------------------------------------------------------
