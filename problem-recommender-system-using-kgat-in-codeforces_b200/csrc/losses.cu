@@ -16,9 +16,9 @@ struct Publish {
     int n_slots;
 };
 
-__global__ void __launch_bounds__(256) loss_reduce_kernel(const float* __restrict__ scratch, int batch, float reg,
-                                                          float* __restrict__ loss, float* __restrict__ loss_sum = nullptr,
-                                                          Publish pub = Publish{nullptr, nullptr, 0}) {
+// run by one block of 256 threads: loss_reduce_kernel, or the last block of transr_reduce_kernel
+__device__ __forceinline__ void loss_reduce(const float* __restrict__ scratch, int batch, float reg, float* __restrict__ loss,
+                                            float* __restrict__ loss_sum, Publish pub) {
     __shared__ float sh_a[8], sh_b[8];
     float a = 0.f, b = 0.f;
     for (int i = threadIdx.x; i < batch; i += 256) {
@@ -48,6 +48,12 @@ __global__ void __launch_bounds__(256) loss_reduce_kernel(const float* __restric
             __threadfence_system();
         }
     }
+}
+
+__global__ void __launch_bounds__(256) loss_reduce_kernel(const float* __restrict__ scratch, int batch, float reg,
+                                                          float* __restrict__ loss, float* __restrict__ loss_sum = nullptr,
+                                                          Publish pub = Publish{nullptr, nullptr, 0}) {
+    loss_reduce(scratch, batch, reg, loss, loss_sum, pub);
 }
 
 inline Publish make_publish(const kgat_publish_t* p) {
@@ -102,63 +108,104 @@ __device__ __forceinline__ int64_t slot_id(const int64_t* __restrict__ a, const 
     return e < batch ? a[e] : (e < 2 * batch ? b[e - batch] : c[e - 2 * batch]);
 }
 
-// Contribution of batch slot k (sample k mod B; role user / positive / negative) to its node's gradient, features [4f, 4f + 4)
-__device__ __forceinline__ void bpr_slot_grad(const float* __restrict__ tab, int64_t ld, const int64_t* __restrict__ users,
-                                              const int64_t* __restrict__ pos, const int64_t* __restrict__ neg, int batch,
-                                              const float* __restrict__ scratch, float g, float lam, int k, int f, float4& acc) {
-    const int b = k % batch, role = k / batch;
-    const float s = sigmoidf_(-scratch[b]) * g;  // d(-logsigmoid(m))/dm = -sigmoid(-m)
-    const float4 a = ldg4(tab + users[b] * ld + f * 4);
-    const float4 x = ldg4(tab + pos[b] * ld + f * 4);
-    const float4 y = ldg4(tab + neg[b] * ld + f * 4);
-    if (role == 0) {
-        acc.x += s * (y.x - x.x) + lam * a.x; acc.y += s * (y.y - x.y) + lam * a.y;
-        acc.z += s * (y.z - x.z) + lam * a.z; acc.w += s * (y.w - x.w) + lam * a.w;
-    } else if (role == 1) {
-        acc.x += -s * a.x + lam * x.x; acc.y += -s * a.y + lam * x.y;
-        acc.z += -s * a.z + lam * x.z; acc.w += -s * a.w + lam * x.w;
+// What the gradient of batch slot k (sample b = k mod B; role user / positive / negative) needs besides table rows: the sample's
+// three ids and s = -d(-logsigmoid(m))/dm * g = sigmoid(-m) g
+struct BprSlot {
+    int64_t u, p, n;
+    float s;
+    int role;
+};
+__device__ __forceinline__ BprSlot bpr_slot(const int64_t* __restrict__ users, const int64_t* __restrict__ pos, const int64_t* __restrict__ neg,
+                                            int batch, const float* __restrict__ scratch, float g, int k) {
+    const int b = k % batch;
+    return BprSlot{users[b], pos[b], neg[b], sigmoidf_(-scratch[b]) * g, k / batch};
+}
+
+// Contribution of one slot to its node's gradient, features [4f, 4f + 4); rounded as nvcc contracts
+// acc += s (y - x) + lam a  (user),  -s a + lam x  (positive),  s a + lam y  (negative)
+__device__ __forceinline__ void bpr_slot_add(const BprSlot& q, const float4& a, const float4& x, const float4& y, float lam, float4& acc) {
+    if (q.role == 0) {
+        acc.x = __fadd_rn(acc.x, __fmaf_rn(lam, a.x, __fmul_rn(q.s, __fsub_rn(y.x, x.x))));
+        acc.y = __fadd_rn(acc.y, __fmaf_rn(lam, a.y, __fmul_rn(q.s, __fsub_rn(y.y, x.y))));
+        acc.z = __fadd_rn(acc.z, __fmaf_rn(lam, a.z, __fmul_rn(q.s, __fsub_rn(y.z, x.z))));
+        acc.w = __fadd_rn(acc.w, __fmaf_rn(lam, a.w, __fmul_rn(q.s, __fsub_rn(y.w, x.w))));
+    } else if (q.role == 1) {
+        acc.x = __fadd_rn(acc.x, __fmaf_rn(lam, x.x, __fmul_rn(-q.s, a.x)));
+        acc.y = __fadd_rn(acc.y, __fmaf_rn(lam, x.y, __fmul_rn(-q.s, a.y)));
+        acc.z = __fadd_rn(acc.z, __fmaf_rn(lam, x.z, __fmul_rn(-q.s, a.z)));
+        acc.w = __fadd_rn(acc.w, __fmaf_rn(lam, x.w, __fmul_rn(-q.s, a.w)));
     } else {
-        acc.x += s * a.x + lam * y.x; acc.y += s * a.y + lam * y.y;
-        acc.z += s * a.z + lam * y.z; acc.w += s * a.w + lam * y.w;
+        acc.x = __fadd_rn(acc.x, __fmaf_rn(lam, y.x, __fmul_rn(q.s, a.x)));
+        acc.y = __fadd_rn(acc.y, __fmaf_rn(lam, y.y, __fmul_rn(q.s, a.y)));
+        acc.z = __fadd_rn(acc.z, __fmaf_rn(lam, y.z, __fmul_rn(q.s, a.z)));
+        acc.w = __fadd_rn(acc.w, __fmaf_rn(lam, y.w, __fmul_rn(q.s, a.w)));
     }
 }
 
 // One warp per id slot e of the batch (users, then positives, then negatives).  The warp of the FIRST slot holding a node
 // sums the contributions of every slot holding it, in slot order, and adds the sum to the node's gradient row: a fixed
-// summation order, so the gradients are bit-identical from run to run (float atomics would add in arrival order).  One pass
-// over the slots decides ownership and lists the node's slots (lane q keeps the q-th); a node held by more than 32 slots
-// rescans them per feature chunk instead.
+// summation order, so the gradients are bit-identical from run to run (float atomics would add in arrival order).  The block
+// stages the slot ids in shared memory; one pass over them decides ownership and lists the node's slots (lane q keeps the
+// q-th and its BprSlot), and the table rows of 4 slots are loaded at once.  A node held by more than 32 slots rescans the ids
+// per feature chunk instead.
+constexpr int kBprIdChunk = 2048;  // slot ids staged per pass (16 KB)
 __global__ void __launch_bounds__(256) bpr_bwd_kernel(Tables T, GradTables G, const int64_t* __restrict__ users,
                                                       const int64_t* __restrict__ pos, const int64_t* __restrict__ neg, int batch,
                                                       float reg, const float* __restrict__ scratch,
                                                       const float* __restrict__ g_loss) {
+    __shared__ int64_t s_ids[kBprIdChunk];
     const int lane = threadIdx.x & 31;
     const int e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int n3 = 3 * batch;
-    if (e >= n3) return;
-    const int64_t id = slot_id(users, pos, neg, batch, e);
+    const int64_t id = e < n3 ? slot_id(users, pos, neg, batch, e) : -1;
+    bool owner = e < n3;
     int my_slot = -1, n_match = 0;
-    for (int k0 = 0; k0 < n3; k0 += 32) {
-        const int k = k0 + lane;
-        const unsigned bal = __ballot_sync(kFull, k < n3 && slot_id(users, pos, neg, batch, k) == id);
-        const unsigned before = e - k0 >= 32 ? kFull : (e > k0 ? (1u << (e - k0)) - 1u : 0u);
-        if (bal & before) return;  // an earlier slot holds the node: its warp owns the row
-        for (unsigned rest = bal; rest; rest &= rest - 1) {
-            const int src = __ffs(rest) - 1;
-            if (n_match + __popc(bal & ((1u << src) - 1u)) == lane) my_slot = k0 + src;
+    for (int c0 = 0; c0 < n3; c0 += kBprIdChunk) {
+        const int cn = n3 - c0 < kBprIdChunk ? n3 - c0 : kBprIdChunk;
+        if (c0 > 0) __syncthreads();
+        for (int t = threadIdx.x; t < cn; t += 256) s_ids[t] = slot_id(users, pos, neg, batch, c0 + t);
+        __syncthreads();
+        for (int k0 = c0; owner && k0 < c0 + cn; k0 += 32) {
+            const int k = k0 + lane;
+            const unsigned bal = __ballot_sync(kFull, k < c0 + cn && s_ids[k - c0] == id);
+            const unsigned before = e - k0 >= 32 ? kFull : (e > k0 ? (1u << (e - k0)) - 1u : 0u);
+            if (bal & before) owner = false;  // an earlier slot holds the node: its warp owns the row
+            for (unsigned rest = bal; rest; rest &= rest - 1) {
+                const int src = __ffs(rest) - 1;
+                if (n_match + __popc(bal & ((1u << src) - 1u)) == lane) my_slot = k0 + src;
+            }
+            n_match += __popc(bal);
         }
-        n_match += __popc(bal);
     }
+    if (!owner) return;
     const float g = g_loss[0] / (float)batch;
     const float lam = reg * g;
+    BprSlot mine{0, 0, 0, 0.f, 0};
+    if (my_slot >= 0) mine = bpr_slot(users, pos, neg, batch, scratch, g, my_slot);
     for (int t = 0; t < T.n; ++t) {
         if (G.p[t] == nullptr) continue;
+        const float* tab = T.p[t];
+        const int64_t ld = T.ld[t];
         for (int f = lane; f - lane < T.q[t]; f += 32) {
             float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
             if (n_match <= 32) {
-                for (int q = 0; q < n_match; ++q) {
-                    const int k = __shfl_sync(kFull, my_slot, q);
-                    if (f < T.q[t]) bpr_slot_grad(T.p[t], T.ld[t], users, pos, neg, batch, scratch, g, lam, k, f, acc);
+                for (int q0 = 0; q0 < n_match; q0 += 4) {
+                    BprSlot sl[4];
+                    float4 a[4], x[4], y[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int src = q0 + u < n_match ? q0 + u : q0;
+                        sl[u] = BprSlot{__shfl_sync(kFull, mine.u, src), __shfl_sync(kFull, mine.p, src), __shfl_sync(kFull, mine.n, src),
+                                        __shfl_sync(kFull, mine.s, src), __shfl_sync(kFull, mine.role, src)};
+                        if (f < T.q[t] && q0 + u < n_match) {
+                            a[u] = ldg4(tab + sl[u].u * ld + f * 4);
+                            x[u] = ldg4(tab + sl[u].p * ld + f * 4);
+                            y[u] = ldg4(tab + sl[u].n * ld + f * 4);
+                        }
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u)
+                        if (f < T.q[t] && q0 + u < n_match) bpr_slot_add(sl[u], a[u], x[u], y[u], lam, acc);
                 }
             } else {
                 for (int k0 = e; k0 < n3; k0 += 32) {
@@ -167,7 +214,10 @@ __global__ void __launch_bounds__(256) bpr_bwd_kernel(Tables T, GradTables G, co
                     while (hits) {
                         const int k = k0 + __ffs(hits) - 1;
                         hits &= hits - 1;
-                        if (f < T.q[t]) bpr_slot_grad(T.p[t], T.ld[t], users, pos, neg, batch, scratch, g, lam, k, f, acc);
+                        if (f < T.q[t]) {
+                            const BprSlot sl = bpr_slot(users, pos, neg, batch, scratch, g, k);
+                            bpr_slot_add(sl, ldg4(tab + sl.u * ld + f * 4), ldg4(tab + sl.p * ld + f * 4), ldg4(tab + sl.n * ld + f * 4), lam, acc);
+                        }
                     }
                 }
             }
@@ -445,22 +495,46 @@ __global__ void __launch_bounds__(128) transr_bwd_kernel(const float* __restrict
 //  * blocks [0, B * D / JB): block (b, jb) -- if sample b is the first of its relation r -- adds the relation's samples' outer
 //    products e^T g_x to rows [JB jb, JB jb + JB) of g_W[r], and block (b, 0) their g_er to g_rel[r].  Warp w takes the samples
 //    i = b + w (mod kRdWarps) in increasing order; the warps' partial sums are combined in warp order;
-//  * the other blocks: one warp per id slot e; the slot that owns its node's compact row (row_slot[node] == e) replaces that
-//    row by the sum of the rows of every slot holding the node, in slot order.
+//  * the next blocks: one warp per id slot e; the slot that owns its node's compact row (row_slot[node] == e) replaces that
+//    row by the sum of the rows of every slot holding the node, in slot order;
+//  * with `loss` set, one last block reduces the loss (loss_reduce): the margins are complete before this launch starts.
+// A warp copies the slices of its next kTrStage<KM> samples into shared memory with cp.async, all in flight at once, before
+// it adds any of them; the id slots are staged in shared memory once per block, and a node's gradient rows are read 4 at a
+// time.  Measured on a B200 at d = 64, B = 512, this takes 5-6 us off the launch when the relations are spread out, but
+// not when one relation holds most of the batch: its 4 blocks take as long as before, so load latency is not their bound.
 constexpr int kRdWarps = 8;
 // rows of g_W[r] per block: the warps' partial sums of the block's JB x K tile plus g_er stay inside 48 KB of shared memory
 __host__ __device__ constexpr int transr_reduce_rows(int d) { return d >= 128 ? 8 : 16; }
+// samples a warp stages at once: the block's staging buffers stay inside 48 KB of shared memory
+template <int KM>
+constexpr int kTrStage = KM == 4 ? 2 : (KM == 2 ? 4 : 8);
+
+__device__ __forceinline__ void cp_async16(float* dst, const float* src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
+}
+// `work` starts 2B floats into the scratch, so its rows are only 8-byte aligned
+__device__ __forceinline__ void cp_async8(float* dst, const float* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory"); }
+
 template <int DM, int KM>
-__global__ void __launch_bounds__(kRdWarps * 32) transr_reduce_kernel(const float* __restrict__ emb, const int64_t* __restrict__ heads,
+__global__ void __launch_bounds__(kRdWarps * 32, DM == 1 ? 4 : 3) transr_reduce_kernel(const float* __restrict__ emb, const int64_t* __restrict__ heads,
                                                                      const int64_t* __restrict__ rels, const int64_t* __restrict__ pt,
                                                                      const int64_t* __restrict__ nt, int batch, const float* __restrict__ work,
                                                                      const int32_t* __restrict__ row_slot, float* __restrict__ g_rows,
-                                                                     float* __restrict__ g_rel, float* __restrict__ g_W) {
+                                                                     float* __restrict__ g_rel, float* __restrict__ g_W,
+                                                                     const float* __restrict__ scratch = nullptr, float reg = 0.f,
+                                                                     float* __restrict__ loss = nullptr, float* __restrict__ loss_sum = nullptr,
+                                                                     Publish pub = Publish{nullptr, nullptr, 0}) {
     constexpr int D = DM * 32, K = KM * 32, JB = transr_reduce_rows(DM * 32), NJB = D / JB, NOUT = JB * K + K;
+    constexpr int S = kTrStage<KM>, SF = 3 * JB + 4 * K;  // per staged sample: e_h, e_p, e_n rows [j0, j0 + JB), then work row
+    constexpr int NBUF = kRdWarps * NOUT > kRdWarps * S * SF ? kRdWarps * NOUT : kRdWarps * S * SF;
+    // staging buffers, then the warps' partial sums (relation blocks); the id slots (row blocks)
+    __shared__ __align__(16) float s_buf[NBUF];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int blk = blockIdx.x;
     if (blk < batch * NJB) {
-        __shared__ float s_part[kRdWarps][NOUT];
         const int b = blk / NJB, jb = blk % NJB, j0 = jb * JB;
         const int64_t r = rels[b];
         int dup = 0;
@@ -473,6 +547,8 @@ __global__ void __launch_bounds__(kRdWarps * 32) transr_reduce_kernel(const floa
 #pragma unroll
             for (int jj = 0; jj < JB; ++jj) acc[jj][m] = 0.f;
         }
+        float* stage = s_buf + warp * S * SF;
+        const int nw2 = (jb == 0 ? 4 : 3) * K / 2;  // 8-byte pieces of a work row this block reads (g_er only in block jb = 0)
         for (int base = b + warp; base < batch; base += kRdWarps * 32) {
             const int il = base + kRdWarps * lane;
             const bool mine = il < batch && rels[il] == r;
@@ -484,28 +560,41 @@ __global__ void __launch_bounds__(kRdWarps * 32) transr_reduce_kernel(const floa
             }
             unsigned hits = __ballot_sync(kFull, mine);
             while (hits) {
-                const int src = __ffs(hits) - 1;
-                hits &= hits - 1;
-                const int i = base + kRdWarps * src;
-                const long long h = __shfl_sync(kFull, hl, src), p = __shfl_sync(kFull, pl, src), n = __shfl_sync(kFull, nl, src);
-                const float* wi = work + (int64_t)i * 4 * K + KM * lane;
-                float ehv[JB], epv[JB], env[JB];
-#pragma unroll
-                for (int c = 0; c < JB; c += 4) {
-                    const float4 a = ldg4(emb + h * D + j0 + c), bq = ldg4(emb + p * D + j0 + c), cq = ldg4(emb + n * D + j0 + c);
-                    ehv[c] = a.x; ehv[c + 1] = a.y; ehv[c + 2] = a.z; ehv[c + 3] = a.w;
-                    epv[c] = bq.x; epv[c + 1] = bq.y; epv[c + 2] = bq.z; epv[c + 3] = bq.w;
-                    env[c] = cq.x; env[c + 1] = cq.y; env[c + 2] = cq.z; env[c + 3] = cq.w;
+                unsigned chunk = hits;  // the warp's next S samples, in increasing order
+                for (int q = 0; q < S && hits; ++q) hits &= hits - 1;
+                chunk &= ~hits;
+                int q = 0;
+                for (unsigned rest = chunk; rest; rest &= rest - 1, ++q) {
+                    const int src = __ffs(rest) - 1;
+                    const long long h = __shfl_sync(kFull, hl, src), p = __shfl_sync(kFull, pl, src), n = __shfl_sync(kFull, nl, src);
+                    float* st = stage + q * SF;
+                    if (lane < 3 * JB / 4) {
+                        const int row = lane / (JB / 4), c = 4 * (lane % (JB / 4));
+                        cp_async16(st + row * JB + c, emb + (row == 0 ? h : (row == 1 ? p : n)) * D + j0 + c);
+                    }
+                    const float* wi = work + (int64_t)(base + kRdWarps * src) * 4 * K;
+                    for (int c = lane; c < nw2; c += 32) cp_async8(st + 3 * JB + 2 * c, wi + 2 * c);
                 }
+                cp_async_wait_all();
+                __syncwarp();
+                for (int qq = 0; qq < q; ++qq) {
+                    const float* ev = stage + qq * SF;
+                    const float* gv = ev + 3 * JB + KM * lane;
 #pragma unroll
-                for (int m = 0; m < KM; ++m) {
-                    const float gh = wi[m], gp = wi[K + m], gn = wi[2 * K + m];
+                    for (int m = 0; m < KM; ++m) {
+                        const float gh = gv[m], gp = gv[K + m], gn = gv[2 * K + m];
+                        // acc += eh gh + ep gp + en gn, rounded as nvcc contracts it: fma(en, gn, fma(eh, gh, ep gp))
 #pragma unroll
-                    for (int jj = 0; jj < JB; ++jj) acc[jj][m] += ehv[jj] * gh + epv[jj] * gp + env[jj] * gn;
-                    if (jb == 0) acc_r[m] += wi[3 * K + m];
+                        for (int jj = 0; jj < JB; ++jj)
+                            acc[jj][m] = __fadd_rn(acc[jj][m], __fmaf_rn(ev[2 * JB + jj], gn, __fmaf_rn(ev[jj], gh, __fmul_rn(ev[JB + jj], gp))));
+                        if (jb == 0) acc_r[m] += gv[3 * K + m];
+                    }
                 }
+                __syncwarp();  // the stage is refilled next
             }
         }
+        __syncthreads();  // s_part overlays the other warps' stages
+        float (*s_part)[NOUT] = reinterpret_cast<float (*)[NOUT]>(s_buf);
 #pragma unroll
         for (int m = 0; m < KM; ++m) {
 #pragma unroll
@@ -524,23 +613,49 @@ __global__ void __launch_bounds__(kRdWarps * 32) transr_reduce_kernel(const floa
         return;
     }
     blk -= batch * NJB;
-    const int n3 = 3 * batch, e = blk * kRdWarps + warp;
-    if (e >= n3) return;
-    const int64_t id = slot_id(heads, pt, nt, batch, e);
-    if (row_slot[id] != e) return;
+    const int n3 = 3 * batch;
+    if (blk * kRdWarps >= n3) {
+        loss_reduce(scratch, batch, reg, loss, loss_sum, pub);
+        return;
+    }
+    const int e = blk * kRdWarps + warp;
+    const int64_t id = e < n3 ? slot_id(heads, pt, nt, batch, e) : -1;
+    const bool owner = e < n3 && row_slot[id] == e;
+    constexpr int CH = NBUF * 4 / 8;  // id slots per staged chunk
+    int64_t* s_ids = reinterpret_cast<int64_t*>(s_buf);
     float acc[DM];
 #pragma unroll
     for (int c = 0; c < DM; ++c) acc[c] = 0.f;
-    for (int k0 = 0; k0 < n3; k0 += 32) {
-        const int kk = k0 + lane;
-        unsigned hits = __ballot_sync(kFull, kk < n3 && slot_id(heads, pt, nt, batch, kk) == id);
-        while (hits) {
-            const int k = k0 + __ffs(hits) - 1;
-            hits &= hits - 1;
+    for (int c0 = 0; c0 < n3; c0 += CH) {
+        const int cn = n3 - c0 < CH ? n3 - c0 : CH;
+        if (c0 > 0) __syncthreads();
+        for (int t = tid; t < cn; t += kRdWarps * 32) s_ids[t] = slot_id(heads, pt, nt, batch, c0 + t);
+        __syncthreads();
+        if (!owner) continue;
+        for (int k0 = 0; k0 < cn; k0 += 32) {
+            unsigned hits = __ballot_sync(kFull, k0 + lane < cn && s_ids[k0 + lane] == id);
+            while (hits) {
+                int ks[4];
 #pragma unroll
-            for (int c = 0; c < DM; ++c) acc[c] += g_rows[(int64_t)k * D + lane + 32 * c];
+                for (int q = 0; q < 4; ++q) {
+                    ks[q] = hits ? c0 + k0 + __ffs(hits) - 1 : -1;
+                    hits &= hits - 1;
+                }
+                float v[4][DM];
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+#pragma unroll
+                    for (int c = 0; c < DM; ++c) v[q][c] = ks[q] >= 0 ? g_rows[(int64_t)ks[q] * D + lane + 32 * c] : 0.f;
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+                    if (ks[q] >= 0) {
+#pragma unroll
+                        for (int c = 0; c < DM; ++c) acc[c] += v[q][c];
+                    }
+            }
         }
     }
+    if (!owner) return;
 #pragma unroll
     for (int c = 0; c < DM; ++c) g_rows[(int64_t)e * D + lane + 32 * c] = acc[c];
 }
@@ -714,13 +829,14 @@ int kgat_transr_step(const float* emb, const float* rel_emb, const float* W, int
     const unsigned blocks = (unsigned)batch;
     // margin[0, 2B): per-sample margin and L2 term; margin[2B, 2B + 4BK): the deterministic backward's work rows
     float* work = margin + 2 * batch;
-    const unsigned reduce_blocks = (unsigned)(batch * (d / transr_reduce_rows(d)) + (3 * batch + kRdWarps - 1) / kRdWarps);
+    // relation blocks, row blocks, one loss block
+    const unsigned reduce_blocks = (unsigned)(batch * (d / transr_reduce_rows(d)) + (3 * batch + kRdWarps - 1) / kRdWarps + 1);
     KGAT_TRANSR_DISPATCH((transr_bwd_kernel<DM, KM, true><<<blocks, 128, 0, stream>>>(emb, rel_emb, W, heads, rels, pos_tails, neg_tails,
                                                                                      batch, reg, margin, nullptr, g_rows, g_rel_emb, g_W,
                                                                                      row_slot, work),
                           transr_reduce_kernel<DM, KM><<<reduce_blocks, kRdWarps * 32, 0, stream>>>(emb, heads, rels, pos_tails, neg_tails, batch, work,
-                                                                                          row_slot, g_rows, g_rel_emb, g_W)));
-    loss_reduce_kernel<<<1, 256, 0, stream>>>(margin, batch, reg, loss, loss_sum, make_publish(publish));
+                                                                                          row_slot, g_rows, g_rel_emb, g_W, margin, reg, loss,
+                                                                                          loss_sum, make_publish(publish))));
     return check_launch();
 }
 
@@ -735,13 +851,14 @@ int kgat_transr_step_claimed(const float* emb, const float* rel_emb, const float
     const unsigned blocks = (unsigned)batch;
     // margin[0, 2B): per-sample margin and L2 term; margin[2B, 2B + 4BK): the deterministic backward's work rows
     float* work = margin + 2 * batch;
-    const unsigned reduce_blocks = (unsigned)(batch * (d / transr_reduce_rows(d)) + (3 * batch + kRdWarps - 1) / kRdWarps);
+    // relation blocks, row blocks, one loss block
+    const unsigned reduce_blocks = (unsigned)(batch * (d / transr_reduce_rows(d)) + (3 * batch + kRdWarps - 1) / kRdWarps + 1);
     KGAT_TRANSR_DISPATCH((transr_bwd_kernel<DM, KM, true><<<blocks, 128, 0, stream>>>(emb, rel_emb, W, heads, rels, pos_tails, neg_tails,
                                                                                      batch, reg, margin, nullptr, g_rows, g_rel_emb, g_W,
                                                                                      row_slot, work),
                           transr_reduce_kernel<DM, KM><<<reduce_blocks, kRdWarps * 32, 0, stream>>>(emb, heads, rels, pos_tails, neg_tails, batch, work,
-                                                                                          row_slot, g_rows, g_rel_emb, g_W)));
-    loss_reduce_kernel<<<1, 256, 0, stream>>>(margin, batch, reg, loss, loss_sum, make_publish(publish));
+                                                                                          row_slot, g_rows, g_rel_emb, g_W, margin, reg, loss,
+                                                                                          loss_sum, make_publish(publish))));
     return check_launch();
 }
 

@@ -488,7 +488,7 @@ def transr_scratch_numel(batch: int, k: int) -> int:
 @_timed("transr_step")
 def transr_step(emb, rel_emb, W, heads, rels, pos_t, neg_t, reg, loss, loss_sum, scratch, row_slot, g_rows, g_rel, g_W, publish=None):
     """Claim compact gradient rows + zero the gradient buffers, TransR forward and backward in one pass, loss value
-    (added to ``loss_sum`` when given): the KG half-step of the epoch engine in four launches."""
+    (added to ``loss_sum`` when given): the KG half-step of the epoch engine in three launches."""
     lib = _lib.load()
     if g_rows.numel() < 3 * heads.numel() * emb.shape[1] or scratch.numel() < transr_scratch_numel(heads.numel(), rel_emb.shape[1]):
         raise KgatLibraryError("transr_step: g_rows needs 3 * batch * d floats, scratch transr_scratch_numel(batch, k)")
