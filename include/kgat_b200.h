@@ -32,7 +32,7 @@ extern "C" {
 #define KGAT_ERR_UNSUPPORTED (-3)
 #define KGAT_ERR_WORKSPACE (-4)
 
-#define KGAT_ABI_VERSION 12
+#define KGAT_ABI_VERSION 13
 #define KGAT_MAX_LAYERS 8   /* embedding table + up to 7 propagation layers */
 #define KGAT_MAX_TENSORS 24 /* tensors per multi-tensor Adam launch */
 #define KGAT_MAX_PEERS 31   /* other ranks of a row-sharded propagation */
@@ -436,6 +436,41 @@ int kgat_rank_targets(const kgat_tables_t* tables, const int32_t* users, int64_t
                       const int32_t* pos_map, int64_t n_pos, const int32_t* target_ptr, const int32_t* target_items, const int64_t* out_ptr,
                       int64_t n_targets, const int32_t* exclude_ptr, const int32_t* exclude_items, int32_t slices, int64_t* out_items,
                       float* out_scores, int64_t* out_rank, int64_t* out_eligible, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------- */
+/* Knowledge-graph completion with the trained TransR half: top-k tails and filtered ranks       */
+/* ------------------------------------------------------------------------------------------- */
+/* Queries (h, r) = (heads[q], rels[q]) (int32 CKG node / relation ids), sorted by relation: segment g holds the queries
+ * seg_ptr_host[g] .. seg_ptr_host[g+1] (host int64 [n_seg + 1], each segment non-empty) of relation seg_rel[g] (device int32
+ * [n_seg]); row q_out[q] of the outputs belongs to query q.  emb [n_nodes, d], rel_emb [n_rel, kdim], W [n_rel, d, kdim]: the
+ * TransR parameters, d = kdim in {32, 64, 128} (KGAT_ERR_UNSUPPORTED otherwise).
+ * Energy E(h, r, t) = ||e_h W_r + e_r - e_t W_r||^2 in fp32, bit-identical to the per-sample term of kgat_transr_forward
+ * (margin = E(h, r, n) - E(h, r, p)).  Key K(q, c) = (float_key(-E) << 32) | (0xFFFFFFFF - c), c = position in cand (int32
+ * node ids, unique); a NaN energy keys as the largest value (ranks first).  ex_keys (nullable): ascending int64 keys
+ * (h n_rel + r) n_nodes + t of known triples; candidate c is not eligible for (h, r) when (h, r, cand[c]) is known.
+ * slices in [0, 64]: candidate slices per 64-query tile (0 = the rule of kgat_recommend_topk; the result does not depend
+ * on it).  Candidate projections are computed for up to 32 relations at a time, within 1 GiB.  Workspace from
+ * kgat_complete_workspace_bytes(d, kdim, n_q, n_tiles, n_cand, n_seg, k, slices, count) with n_tiles = sum over segments of
+ * ceil(size / 64) and count = 1 for kgat_complete_rank (k ignored), 0 for kgat_complete_topk; -1 for invalid arguments.
+ * No host synchronisation. */
+int64_t kgat_complete_workspace_bytes(int32_t d, int32_t kdim, int64_t n_queries, int64_t n_tiles, int64_t n_cand, int32_t n_rel_used, int32_t k,
+                                      int32_t slices, int32_t count);
+/* Top-k eligible tails per query, lowest energy first: out_tails int64 [n_q, k] (node ids, -1 after out_count[row]),
+ * out_energy fp32 [n_q, k] (+inf after out_count[row]), out_count int32 [n_q] = min(k, eligible candidates); k in [1, 128]. */
+int kgat_complete_topk(const float* emb, const float* rel_emb, const float* W, int32_t d, int32_t kdim, int64_t n_nodes, int64_t n_rel,
+                       const int32_t* heads, const int32_t* rels, const int32_t* q_out, int64_t n_q, const int64_t* seg_ptr_host,
+                       const int32_t* seg_rel, int32_t n_seg, const int32_t* cand, int64_t n_cand, const int64_t* ex_keys, int64_t n_ex,
+                       int32_t k, int32_t slices, int64_t* out_tails, float* out_energy, int32_t* out_count, void* workspace,
+                       int64_t workspace_bytes, void* stream);
+/* Filtered rank of the target tails[q]: out_rank int64 [n_q] = #{eligible c != t : K(q, c) > K(q, t)} (the target stays
+ * eligible even when (h, r, t) is known), -1 when t is not a candidate; out_energy fp32 [n_q] = E(h, r, t); out_eligible int64
+ * [n_q] = candidates not known for (h, r), the target counted.  pos_map (nullable): int32 [n_nodes], position of a node in
+ * cand or -1; NULL means cand[c] == c. */
+int kgat_complete_rank(const float* emb, const float* rel_emb, const float* W, int32_t d, int32_t kdim, int64_t n_nodes, int64_t n_rel,
+                       const int32_t* heads, const int32_t* rels, const int32_t* tails, const int32_t* q_out, int64_t n_q,
+                       const int64_t* seg_ptr_host, const int32_t* seg_rel, int32_t n_seg, const int32_t* cand, int64_t n_cand,
+                       const int32_t* pos_map, const int64_t* ex_keys, int64_t n_ex, int32_t slices, float* out_energy, int64_t* out_rank,
+                       int64_t* out_eligible, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* K11: Adam                               reference model.py:393-419 (torch.optim.Adam)       */

@@ -208,6 +208,84 @@ inline int pick_slices(int64_t n_users, int64_t n_cand_max, int per_sm, int requ
     return (int)(s < 1 ? 1 : s);
 }
 
+// ------------------------------------------------------------------------------------------
+// Running top-k lists of the fused selection kernels (recommend.cu, complete.cu): an entry is a value and a candidate index,
+// ordered by descending float_key(value), then ascending index -- a total order, so a list does not depend on how the
+// candidates were split.  k <= kTopkMaxK; a CTA folds at most kTileItems pending entries per row at a time.
+// ------------------------------------------------------------------------------------------
+constexpr int kTopkMaxK = 128;  // = kTopkMax of topk_rows
+
+struct Entry {
+    float s;
+    int c;  // candidate index
+};
+
+// true when a ranks before b
+__device__ __forceinline__ bool beats(const Entry& a, const Entry& b) {
+    const uint32_t ka = float_key(a.s), kb = float_key(b.s);
+    return ka != kb ? ka > kb : a.c < b.c;
+}
+
+// number of entries of the sorted list l[0, n) that beat x
+__device__ __forceinline__ int count_beating(const Entry* l, int n, const Entry& x) {
+    int lo = 0;
+    while (n > 0) {
+        const int half = n >> 1;
+        if (beats(l[lo + half], x)) {
+            lo += half + 1;
+            n -= half + 1;
+        } else {
+            n = half;
+        }
+    }
+    return lo;
+}
+
+// One warp folds the np <= kTileItems unordered entries pl into the sorted list tl[0, nt): rank = members of the union that
+// beat it.  Returns the new length min(nt + np, k).
+__device__ __forceinline__ int fold_pending(Entry* tl, int nt, const Entry* pl, int np, int k, int lane) {
+    constexpr int M = (kTopkMaxK + kTileItems) / 32;
+    const int n_union = nt + np;
+    Entry xs[M];
+    int rk[M];
+#pragma unroll
+    for (int m = 0; m < M; ++m) {
+        const int e = lane + 32 * m;
+        rk[m] = k;
+        if (e < n_union) {
+            const Entry x = e < nt ? tl[e] : pl[e - nt];
+            int r = e < nt ? e : count_beating(tl, nt, x);
+            for (int j = 0; j < np && r < k; ++j) r += beats(pl[j], x);
+            xs[m] = x;
+            rk[m] = r;
+        }
+    }
+    __syncwarp();
+#pragma unroll
+    for (int m = 0; m < M; ++m)
+        if (rk[m] < k) tl[rk[m]] = xs[m];
+    __syncwarp();
+    return n_union < k ? n_union : k;
+}
+
+// One warp merges a row's per-slice sorted lists (lists[s * k ..], lens[s]) by rank: put(r, x) for every entry x of merged
+// rank r < k.  Returns min(k, total entries).
+template <class Put>
+__device__ __forceinline__ int merge_slices(const Entry* lists, const int32_t* lens, int slices, int k, int lane, Put put) {
+    int total = 0;
+    for (int s = 0; s < slices; ++s) total += lens[s];
+    for (int e = lane; e < slices * k; e += 32) {
+        const int s = e / k, i = e % k;
+        if (i >= lens[s]) continue;
+        const Entry x = lists[e];
+        int r = i;
+        for (int v = 0; v < slices && r < k; ++v)
+            if (v != s) r += count_beating(lists + v * k, lens[v], x);
+        if (r < k) put(r, x);
+    }
+    return total < k ? total : k;
+}
+
 // log(sigmoid(x)) as ATen computes it: min(x,0) - log1p(exp(-|x|))
 __device__ __forceinline__ float log_sigmoid(float x) { return fminf(x, 0.f) - log1pf(expf(-fabsf(x))); }
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }

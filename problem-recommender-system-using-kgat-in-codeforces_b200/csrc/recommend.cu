@@ -21,34 +21,8 @@ namespace {
 constexpr int kRecThreads = kTileThreads;
 constexpr int kRecUsers = kTileUsers;  // users per CTA
 constexpr int kRecItems = kTileItems;  // candidates per tile
-constexpr int kRecMaxK = 128;          // = kTopkMax of topk_rows
+constexpr int kRecMaxK = kTopkMaxK;
 constexpr int kRecMaxSlices = kTileMaxSlices;
-
-struct Entry {
-    float s;
-    int c;  // candidate index
-};
-
-// true when a ranks before b
-__device__ __forceinline__ bool beats(const Entry& a, const Entry& b) {
-    const uint32_t ka = float_key(a.s), kb = float_key(b.s);
-    return ka != kb ? ka > kb : a.c < b.c;
-}
-
-// number of entries of the sorted list l[0, n) that beat x
-__device__ __forceinline__ int count_beating(const Entry* l, int n, const Entry& x) {
-    int lo = 0;
-    while (n > 0) {
-        const int half = n >> 1;
-        if (beats(l[lo + half], x)) {
-            lo += half + 1;
-            n -= half + 1;
-        } else {
-            n = half;
-        }
-    }
-    return lo;
-}
 
 inline int64_t align256(int64_t b) { return (b + 255) & ~int64_t(255); }
 
@@ -200,29 +174,9 @@ __global__ void __launch_bounds__(kRecThreads) recommend_score_kernel(ScoreArgs 
         for (int ul = warp; ul < kRecUsers; ul += kRecThreads / 32) {
             const int np = n_pend[ul];
             if (np == 0) continue;
-            const int nt = n_top[ul], n_union = nt + np;
-            Entry* tl = top + ul * k;
-            const Entry* pl = pend + ul * kRecItems;
-            Entry xs[(kRecMaxK + kRecItems) / 32];
-            int rk[(kRecMaxK + kRecItems) / 32];
-#pragma unroll
-            for (int m = 0; m < (kRecMaxK + kRecItems) / 32; ++m) {
-                const int e = lane + 32 * m;
-                rk[m] = k;
-                if (e < n_union) {
-                    const Entry x = e < nt ? tl[e] : pl[e - nt];
-                    int r = e < nt ? e : count_beating(tl, nt, x);
-                    for (int j = 0; j < np && r < k; ++j) r += beats(pl[j], x);
-                    xs[m] = x;
-                    rk[m] = r;
-                }
-            }
-            __syncwarp();
-#pragma unroll
-            for (int m = 0; m < (kRecMaxK + kRecItems) / 32; ++m)
-                if (rk[m] < k) tl[rk[m]] = xs[m];
+            const int n_new = fold_pending(top + ul * k, n_top[ul], pend + ul * kRecItems, np, k, lane);
             if (lane == 0) {
-                n_top[ul] = n_union < k ? n_union : k;
+                n_top[ul] = n_new;
                 n_pend[ul] = 0;
             }
             __syncwarp();
@@ -246,23 +200,10 @@ __global__ void __launch_bounds__(256) recommend_merge_kernel(const Entry* __res
     const int lane = threadIdx.x & 31;
     const int64_t u = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     if (u >= n_users) return;
-    const Entry* lists = ws_list + u * slices * k;
-    const int32_t* lens = ws_len + u * slices;
-    int total = 0;
-    for (int s = 0; s < slices; ++s) total += lens[s];
-    if (total > k) total = k;
-    for (int e = lane; e < slices * k; e += 32) {
-        const int s = e / k, i = e % k;
-        if (i >= lens[s]) continue;
-        const Entry x = lists[e];
-        int r = i;
-        for (int v = 0; v < slices && r < k; ++v)
-            if (v != s) r += count_beating(lists + v * k, lens[v], x);
-        if (r < k) {
-            out_items[u * k + r] = cand[x.c];
-            out_scores[u * k + r] = x.s;
-        }
-    }
+    const int total = merge_slices(ws_list + u * slices * k, ws_len + u * slices, slices, k, lane, [&](int r, const Entry& x) {
+        out_items[u * k + r] = cand[x.c];
+        out_scores[u * k + r] = x.s;
+    });
     for (int r = total + lane; r < k; r += 32) {
         out_items[u * k + r] = -1;
         out_scores[u * k + r] = -INFINITY;

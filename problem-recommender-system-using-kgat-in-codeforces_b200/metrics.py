@@ -190,3 +190,105 @@ def rank_metrics(model, train: InteractionCSR, test: InteractionCSR, k_list=(20,
     out: dict = {k: dict(zip(("precision", "recall", "ndcg", "hit"), vals[4 * j : 4 * j + 4])) for j, k in enumerate(k_list)}
     out.update(zip(("mrr", "auc", "mean_rank"), vals[4 * len(k_list) :]))
     return out
+
+
+class TripleSet:
+    """A set of CKG triples ``(h, r, t)`` as sorted unique int64 keys ``(h * relation_num + r) * node_num + t`` on the device:
+    the known triples of the filtered link-prediction protocol (``KGAT.complete`` / ``KGAT.kg_rank`` ``exclude``)."""
+
+    def __init__(self, heads, relations, tails, node_num: int, relation_num: int, device):
+        node_num, relation_num = int(node_num), int(relation_num)
+        if node_num < 1 or relation_num < 1:
+            raise ValueError("node_num and relation_num must be positive")
+        if node_num * node_num * relation_num > np.iinfo(np.int64).max:
+            raise ValueError(f"keys of {node_num} nodes and {relation_num} relations do not fit int64")
+        cols = [torch.as_tensor(x).to(device=device, dtype=torch.int64).flatten() for x in (heads, relations, tails)]
+        if not cols[0].numel() == cols[1].numel() == cols[2].numel():
+            raise ValueError("heads, relations and tails differ in length")
+        h, r, t = cols
+        if h.numel():
+            lo = torch.stack([h.min(), r.min(), t.min()]).min()
+            hi_h, hi_r, hi_t = torch.stack([h.max(), r.max(), t.max()]).tolist()
+            if int(lo) < 0 or hi_h >= node_num or hi_t >= node_num or hi_r >= relation_num:
+                raise ValueError(f"triples must hold node ids in [0, {node_num}) and relation ids in [0, {relation_num})")
+        self.node_num, self.relation_num = node_num, relation_num
+        self.keys = torch.unique((h * relation_num + r) * node_num + t)  # sorted
+
+    @classmethod
+    def from_ckg(cls, g, device="cuda") -> "TripleSet":
+        """Every triple of the CKG edge list (``g.heads / relations / tails``): what TransR trains on."""
+        return cls(torch.from_numpy(np.asarray(g.heads)), torch.from_numpy(np.asarray(g.relations)), torch.from_numpy(np.asarray(g.tails)),
+                   g.node_num, g.relation_num, device)
+
+    def __len__(self) -> int:
+        return int(self.keys.numel())
+
+    def triples(self):
+        """(heads, relations, tails) int64 on the device, in key order."""
+        t = self.keys % self.node_num
+        hr = self.keys // self.node_num
+        return hr // self.relation_num, hr % self.relation_num, t
+
+
+def link_terms(rank: torch.Tensor, hits) -> torch.Tensor:
+    """Per-query fp64 terms [Q, 3 + len(hits)] of the filtered link-prediction metrics from 0-based ranks (-1 = not ranked):
+    ranked flag, 1 / (rank + 1), rank + 1, then [rank < k] for every k of ``hits``; zeros for unranked queries."""
+    ok = rank >= 0
+    r1 = (rank + 1).to(torch.float64)
+    cols = [ok.to(torch.float64), torch.where(ok, 1.0 / r1, 0.0), torch.where(ok, r1, 0.0)]
+    cols += [(ok & (rank < k)).to(torch.float64) for k in hits]
+    return torch.stack(cols, 1)
+
+
+@torch.no_grad()
+def link_metrics(model, triples, known, hits=(1, 3, 10), candidates="relation") -> dict:
+    """Filtered link prediction of the trained TransR half: the rank of each held-out triple's tail (``KGAT.kg_rank``) among the
+    candidates, with every other triple of ``known`` (a ``TripleSet``) filtered out (Bordes et al. 2013).
+
+    ``triples``: a ``TripleSet`` or ``(heads, relations, tails)`` of the triples to rank.  ``candidates``: ``"relation"`` -- the
+    tail nodes of the query's relation in ``known`` (type-constrained), ``"all"`` -- every CKG node, or a 1-D tensor of node
+    ids.  Head prediction needs no second call: every CKG relation has its inverse in the edge list.  Queries are grouped by
+    relation, one ``kg_rank`` call per relation; per-query terms are fp64 on the device, summed in a fixed order and read back
+    once.  A triple whose tail is not a candidate is skipped (``n_skipped``).
+
+    Returns ``{"mrr", "mean_rank" (1-based), "hits": {k: ...}, "per_relation": {r: {"mrr", "mean_rank", "hits", "n_ranked"}},
+    "n_ranked", "n_skipped"}``; means over the ranked queries (NaN when there is none)."""
+    hits = [int(k) for k in hits]
+    if not hits or min(hits) < 1:
+        raise ValueError(f"hits must hold positive ints, got {hits}")
+    dev = model._device()
+    N, R = model.node_num, model._relation_num
+    if known.node_num != N or known.relation_num != R:
+        raise ValueError(f"known is a TripleSet over {known.node_num} nodes and {known.relation_num} relations, the model has {N} and {R}")
+    if isinstance(triples, TripleSet):
+        h, r, t = triples.triples()
+    else:
+        h, r, t = (torch.as_tensor(x).to(device=dev, dtype=torch.int64).flatten() for x in triples)
+    if isinstance(candidates, str) and candidates not in ("relation", "all"):
+        raise ValueError(f'candidates must be "relation", "all" or a tensor of node ids, got {candidates!r}')
+    rels = torch.unique(r).tolist()
+    if rels and (rels[0] < 0 or rels[-1] >= R):
+        raise ValueError(f"relation ids must lie in [0, {R})")
+    if isinstance(candidates, str) and candidates == "relation":
+        _, kr, kt = known.triples()
+    sums, per = [], []
+    for rel in rels:
+        sel = torch.nonzero(r == rel).flatten()
+        if isinstance(candidates, str):
+            cand = N if candidates == "all" else torch.unique(kt[kr == rel])
+        else:
+            cand = candidates
+        ranks = model.kg_rank(h[sel], r[sel], t[sel], cand, exclude=known)
+        per.append(link_terms(ranks.rank, hits).sum(0))
+    terms = torch.stack(per) if per else torch.zeros(0, 3 + len(hits), dtype=torch.float64, device=dev)
+    vals = torch.cat([terms, terms.sum(0, keepdim=True)]).tolist()  # rows: relations in ascending id, then the total
+
+    def summary(v):
+        n = v[0]
+        div = (lambda x: x / n) if n > 0 else (lambda x: float("nan"))
+        return {"mrr": div(v[1]), "mean_rank": div(v[2]), "hits": {k: div(v[3 + j]) for j, k in enumerate(hits)}, "n_ranked": int(n)}
+
+    total = summary(vals[-1])
+    return {"mrr": total["mrr"], "mean_rank": total["mean_rank"], "hits": total["hits"],
+            "per_relation": {rel: summary(v) for rel, v in zip(rels, vals[:-1])}, "n_ranked": total["n_ranked"],
+            "n_skipped": int(h.numel()) - total["n_ranked"]}

@@ -88,6 +88,25 @@ class TargetRanks:
     eligible: torch.Tensor  # int64 [U]: number of eligible problems of the user
 
 
+@dataclass
+class Completion:
+    """Result of ``KGAT.complete`` for Q queries ``(h, r, ?)``: each query's top-k eligible tails, lowest TransR energy first.
+    Positions from ``count`` on hold tail -1 and energy +inf."""
+
+    tails: torch.Tensor  # int64 [Q, k]: CKG node ids
+    energy: torch.Tensor  # fp32 [Q, k]: ||e_h W_r + e_r - e_t W_r||^2, bit-identical to the TransR loss's term
+    count: torch.Tensor  # int32 [Q]: min(k, number of eligible candidates)
+
+
+@dataclass
+class TailRanks:
+    """Result of ``KGAT.kg_rank`` for Q triples ``(h, r, t)``."""
+
+    energy: torch.Tensor  # fp32 [Q]: the TransR energy of the triple
+    rank: torch.Tensor  # int64 [Q]: eligible candidates ranked before t (0 = first), -1 when t is not a candidate
+    eligible: torch.Tensor  # int64 [Q]: number of eligible candidates, t included
+
+
 class KGATMode(IntEnum):
     TRAIN_CF = 0
     TRAIN_KG = 1
@@ -705,6 +724,80 @@ class KGAT(nn.Module):
         ptr, t, scores, rank, eligible = ops.launch_rank(tables, users32, cand32, t_ptr, t_items, out_ptr, n_targets, ex_ptr, ex_items,
                                                          arange=isinstance(items, int), n_pos=self._entity_num)
         return TargetRanks(ptr=ptr, items=t, scores=scores, rank=rank, eligible=eligible)
+
+    def _transr_params(self):
+        """The trained TransR half (entity table after settling deferred KG rows, relation embeddings, projections), read without
+        invalidating any cache or captured step."""
+        self._settle()
+        return self._emb_raw().detach(), self._relation_embedding._parameters["weight"].detach(), self._trans_matrix.detach()
+
+    @staticmethod
+    def _exclude_keys(exclude, node_num: int, relation_num: int):
+        if exclude is None:
+            return None
+        if exclude.node_num != node_num or exclude.relation_num != relation_num:
+            raise ValueError(f"exclude is a TripleSet over {exclude.node_num} nodes and {exclude.relation_num} relations, the model has "
+                             f"{node_num} and {relation_num}")
+        return exclude.keys
+
+    @torch.no_grad()
+    def complete(self, heads, relations, candidates, k: int = 10, exclude=None) -> "Completion":
+        """Knowledge-graph completion with the trained TransR half: for every query ``(heads[q], relations[q], ?)`` the ``k`` most
+        plausible tails among ``candidates``, in one call, without an energy matrix.
+
+        ``heads`` / ``relations``: 1-D int32 / int64 CKG node ids in ``[0, node_num)`` and relation ids in ``[0, relation_num)``
+        -- the ids of ``CKG.heads / relations / tails``, the triples TransR trains on.  The edge list holds each relation's
+        inverse, so "which rating has problem p" is the query ``(user_num + p, r)`` with ``r`` the inverse of the rating
+        relation.  ``candidates``: an int ``n`` (= ``arange(n)``) or a 1-D tensor of unique node ids; its order breaks ties.
+        ``exclude``: ``None`` or a ``metrics.TripleSet`` of known triples; ``c`` is not returned for ``(h, r)`` when ``(h, r, c)``
+        is in it (the filtered protocol).
+
+        Energy ``E(h, r, t) = ||e_h W_r + e_r - e_t W_r||^2`` in fp32, bit-identical to the per-sample term of the TransR loss.
+        Order: energy ascending (the key ``float_key(-E)`` of ``recommend``'s order; a NaN energy first), then earlier position
+        in ``candidates``.  ``1 <= k <= 128``; queries with fewer than ``k`` eligible candidates get ``count < k`` and -1 / +inf
+        padding.
+
+        Settles deferred KG rows and reads the parameters only: no cache or captured step is invalidated and no RNG is drawn,
+        so calling it between training steps leaves training unchanged.  ValueError for every malformed argument.  One host
+        synchronisation (the range-check read-back)."""
+        self._device()
+        emb, rel, w = self._transr_params()
+        ex = self._exclude_keys(exclude, self.node_num, self._relation_num)
+        tails, energy, count = ops.complete_topk(emb, rel, w, self._query_ids(heads, "heads"), self._query_ids(relations, "relations"),
+                                                 self._candidates(candidates), k, ex)
+        return Completion(tails=tails, energy=energy, count=count)
+
+    @torch.no_grad()
+    def kg_rank(self, heads, relations, tails, candidates, exclude=None) -> "TailRanks":
+        """The filtered rank of each triple's tail among ``candidates``: link prediction for the trained TransR half.
+
+        Arguments as for ``complete``; ``tails``: 1-D node ids of the same length.  A candidate ``c`` is eligible for
+        ``(h, r, t)`` when ``(h, r, c)`` is not in ``exclude`` or ``c == t`` (the target itself stays eligible).  With ``complete``'s
+        key ``K``::
+
+            rank(q) = #{c eligible, c != t : K(q, c) > K(q, t)}
+
+        so ``rank < k`` means ``complete(..., k, exclude minus (h, r, t)).tails[q, rank] == t``.  -1 when ``t`` is not in
+        ``candidates``.  ``energy`` is ``E(h, r, t)`` in any case, and ``energy(h, r, n) - energy(h, r, p)`` is the TransR loss's
+        margin bit for bit.  Only integers are counted, so the result does not depend on how the GPU splits the work.  Reads
+        parameters only, as ``complete``; one host synchronisation."""
+        self._device()
+        emb, rel, w = self._transr_params()
+        ex = self._exclude_keys(exclude, self.node_num, self._relation_num)
+        energy, rank, eligible = ops.kg_rank(emb, rel, w, self._query_ids(heads, "heads"), self._query_ids(relations, "relations"),
+                                             self._query_ids(tails, "tails"), self._candidates(candidates), ex)
+        return TailRanks(energy=energy, rank=rank, eligible=eligible)
+
+    def _query_ids(self, ids, name: str) -> torch.Tensor:
+        t = torch.as_tensor(ids)
+        if t.dim() != 1 or t.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f"{name} must be a 1-D int32 / int64 tensor, got {t.dtype} of shape {tuple(t.shape)}")
+        return t.to(device=self._device(), dtype=torch.int64)
+
+    def _candidates(self, candidates):
+        if isinstance(candidates, bool) or not isinstance(candidates, (int, torch.Tensor)):
+            raise ValueError("candidates must be an int or a 1-D int32 / int64 tensor of node ids")
+        return candidates if isinstance(candidates, int) else self._query_ids(candidates, "candidates")
 
     @torch.no_grad()
     def explain(self, user_ids, item_ids, k: int = 10, max_hops: int | None = None) -> "PathExplanation":

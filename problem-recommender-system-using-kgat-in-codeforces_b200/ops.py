@@ -937,6 +937,113 @@ def launch_rank(tables, users32: torch.Tensor, cand32: torch.Tensor, target_ptr,
     return out_ptr, items, scores, rank, eligible
 
 
+def _completion_queries(emb, rel_emb, W, heads, rels, tails, candidates, exclude_keys, slices):
+    """Shared checks of ``complete_topk`` / ``kg_rank``; the queries sorted by relation (stable) and one read-back of the ranges,
+    duplicates and per-relation query counts.  Returns a dict of what the launch needs."""
+    if slices is not None and not 1 <= int(slices) <= 64:
+        raise ValueError(f"slices must be in [1, 64], got {slices}")
+    if emb.dim() != 2 or rel_emb.dim() != 2 or W.dim() != 3 or W.shape != (rel_emb.shape[0], emb.shape[1], rel_emb.shape[1]):
+        raise ValueError("emb [N, d], rel_emb [R, k] and W [R, d, k] do not fit together")
+    N, R = emb.shape[0], rel_emb.shape[0]
+    if not (emb.shape[1] == rel_emb.shape[1] and emb.shape[1] in (32, 64, 128)):
+        raise KgatLibraryError(f"complete: TransR widths d = {emb.shape[1]}, k = {rel_emb.shape[1]} unsupported (d = k in 32, 64, 128)")
+    dev = emb.device
+    heads, rels = _ids64(heads, "heads", dev), _ids64(rels, "relations", dev)
+    if heads.numel() != rels.numel() or (tails is not None and tails.numel() != heads.numel()):
+        raise ValueError("heads, relations (and tails) differ in length")
+    arange = isinstance(candidates, int)
+    if arange and not 0 <= candidates <= N:
+        raise ValueError(f"candidates = {candidates} must lie in [0, {N}]")
+    if not arange and not isinstance(candidates, torch.Tensor):
+        raise ValueError("candidates must be an int or a 1-D integer tensor of node ids")
+    cand = torch.arange(candidates, device=dev) if arange else _ids64(candidates, "candidates", dev)
+    if exclude_keys is not None and (exclude_keys.dim() != 1 or exclude_keys.dtype != i64 or exclude_keys.device != dev):
+        raise ValueError("exclude must hold int64 keys on the parameters' device")
+    order = torch.sort(rels, stable=True).indices
+    counts = torch.zeros(R, dtype=i64, device=dev).index_add_(0, rels.clamp(0, R - 1), torch.ones_like(rels))
+    checks = [("head ids", heads, N), ("relation ids", rels, R), ("candidate ids", cand, N)]
+    if tails is not None:
+        checks.append(("tail ids", _ids64(tails, "tails", dev), N))
+    got = range_check(checks, dev, flags=[("candidates hold duplicate ids", duplicate_count(cand))], values=list(counts))
+    ids = [got[j][order].contiguous() if j != 2 else None for j in range(len(checks))]  # the queries in sorted order
+    counts = got[len(checks) :]
+    seg_rel = [r for r in range(R) if counts[r] > 0]
+    seg_ptr = [0]
+    for r in seg_rel:
+        seg_ptr.append(seg_ptr[-1] + counts[r])
+    pos_map = None
+    if tails is not None and not arange:
+        pos_map = torch.full((N,), -1, dtype=i32, device=dev)
+        pos_map[got[2].long()] = torch.arange(got[2].numel(), dtype=i32, device=dev)
+    ex = exclude_keys if exclude_keys is not None and exclude_keys.numel() else None
+    return dict(N=N, R=R, d=emb.shape[1], kdim=rel_emb.shape[1], heads=ids[0], rels=ids[1], cand=got[2], tails=ids[3] if tails is not None else None,
+                q_out=order.to(i32), seg_rel=torch.tensor(seg_rel, dtype=i32, device=dev), seg_ptr=seg_ptr,
+                n_tiles=sum((seg_ptr[g + 1] - seg_ptr[g] + 63) // 64 for g in range(len(seg_rel))), pos_map=pos_map, ex=ex,
+                slices=0 if slices is None else int(slices))
+
+
+def _completion_workspace(q, k: int, count: bool):
+    lib = _lib.load()
+    ws_bytes = int(lib.kgat_complete_workspace_bytes(q["d"], q["kdim"], q["heads"].numel(), q["n_tiles"], q["cand"].numel(), len(q["seg_ptr"]) - 1,
+                                                     k, q["slices"], int(count)))
+    if ws_bytes < 0:
+        raise KgatLibraryError(f"complete: width {q['kdim']} rejected (too wide for shared memory at k = {k})")
+    return torch.empty(max(ws_bytes, 1), dtype=u8, device=q["heads"].device), ws_bytes
+
+
+def complete_topk(emb, rel_emb, W, heads, rels, candidates, k: int, exclude_keys=None, slices=None):
+    """Top-``k`` tails of the queries ``(heads[q], rels[q], ?)`` among ``candidates`` under the TransR parameters, lowest energy
+    first, without an energy matrix (``kgat_complete_topk``).  ``emb`` [N, d] / ``rel_emb`` [R, k] / ``W`` [R, d, k]: the
+    entity table, relation embeddings and projection matrices; ``heads`` / ``rels``: 1-D ids, any integer dtype;
+    ``candidates``: an int ``n`` (= ``arange(n)``) or 1-D unique node ids, whose order breaks energy ties;
+    ``exclude_keys``: ``metrics.TripleSet.keys`` of known triples (not returned).  ``slices`` (1 .. 64, None = automatic) does
+    not change the result.  One host synchronisation.  Returns ``(tails int64 [Q, k], energy fp32 [Q, k], count int32 [Q])``
+    padded with -1 / +inf after ``count``."""
+    k = int(k)
+    if not 1 <= k <= 128:
+        raise ValueError(f"k must be in [1, 128], got {k}")
+    q = _completion_queries(emb, rel_emb, W, heads, rels, None, candidates, exclude_keys, slices)
+    dev, Q = emb.device, q["heads"].numel()
+    tails = torch.empty(Q, k, dtype=i64, device=dev)
+    energy = torch.empty(Q, k, dtype=f32, device=dev)
+    count = torch.empty(Q, dtype=i32, device=dev)
+    if Q == 0:
+        return tails, energy, count
+    ws, ws_bytes = _completion_workspace(q, k, False)
+    seg_ptr = (C.c_int64 * len(q["seg_ptr"]))(*q["seg_ptr"])
+    n = q["cand"].numel()
+    check(_lib.load().kgat_complete_topk(
+        _ptr(emb, f32, "emb"), _ptr(rel_emb, f32, "rel_emb"), _ptr(W, f32, "W"), q["d"], q["kdim"], q["N"], q["R"], q["heads"].data_ptr(),
+        q["rels"].data_ptr(), q["q_out"].data_ptr(), Q, seg_ptr, q["seg_rel"].data_ptr(), len(q["seg_ptr"]) - 1, q["cand"].data_ptr() if n else None,
+        n, None if q["ex"] is None else q["ex"].data_ptr(), 0 if q["ex"] is None else q["ex"].numel(), k, q["slices"], tails.data_ptr(),
+        energy.data_ptr(), count.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "complete_topk")
+    return tails, energy, count
+
+
+def kg_rank(emb, rel_emb, W, heads, rels, tails, candidates, exclude_keys=None, slices=None):
+    """Filtered rank of the tail of every triple ``(heads[q], rels[q], tails[q])`` among ``candidates`` (``kgat_complete_rank``):
+    ``rank`` = the eligible candidates other than the target whose (energy, position) key beats the target's, -1 when the
+    target is not a candidate; the target stays eligible when its own triple is in ``exclude_keys``.  Arguments as for
+    ``complete_topk``.  One host synchronisation.  Returns ``(energy fp32 [Q], rank int64 [Q], eligible int64 [Q])``."""
+    q = _completion_queries(emb, rel_emb, W, heads, rels, tails, candidates, exclude_keys, slices)
+    dev, Q = emb.device, q["heads"].numel()
+    energy = torch.empty(Q, dtype=f32, device=dev)
+    rank = torch.empty(Q, dtype=i64, device=dev)
+    eligible = torch.empty(Q, dtype=i64, device=dev)
+    if Q == 0:
+        return energy, rank, eligible
+    ws, ws_bytes = _completion_workspace(q, 1, True)
+    seg_ptr = (C.c_int64 * len(q["seg_ptr"]))(*q["seg_ptr"])
+    n = q["cand"].numel()
+    check(_lib.load().kgat_complete_rank(
+        _ptr(emb, f32, "emb"), _ptr(rel_emb, f32, "rel_emb"), _ptr(W, f32, "W"), q["d"], q["kdim"], q["N"], q["R"], q["heads"].data_ptr(),
+        q["rels"].data_ptr(), q["tails"].data_ptr(), q["q_out"].data_ptr(), Q, seg_ptr, q["seg_rel"].data_ptr(), len(q["seg_ptr"]) - 1,
+        q["cand"].data_ptr() if n else None, n, None if q["pos_map"] is None else q["pos_map"].data_ptr(),
+        None if q["ex"] is None else q["ex"].data_ptr(), 0 if q["ex"] is None else q["ex"].numel(), q["slices"], energy.data_ptr(),
+        rank.data_ptr(), eligible.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "kg_rank")
+    return energy, rank, eligible
+
+
 # ----------------------------------------------------------------------------------------------
 # K11 Adam
 # ----------------------------------------------------------------------------------------------
