@@ -32,7 +32,7 @@ extern "C" {
 #define KGAT_ERR_UNSUPPORTED (-3)
 #define KGAT_ERR_WORKSPACE (-4)
 
-#define KGAT_ABI_VERSION 13
+#define KGAT_ABI_VERSION 14
 #define KGAT_MAX_LAYERS 8   /* embedding table + up to 7 propagation layers */
 #define KGAT_MAX_TENSORS 24 /* tensors per multi-tensor Adam launch */
 #define KGAT_MAX_PEERS 31   /* other ranks of a row-sharded propagation */
@@ -412,6 +412,34 @@ int64_t kgat_recommend_workspace_bytes(const kgat_tables_t* tables, int64_t n_us
 int kgat_recommend_topk(const kgat_tables_t* tables, const int32_t* users, int64_t n_users, const int32_t* cand_items, int64_t n_cand_max,
                         const int32_t* n_cand, int32_t k, const int32_t* exclude_ptr, const int32_t* exclude_items, int32_t slices,
                         int64_t* out_items, float* out_scores, int32_t* out_count, void* workspace, int64_t workspace_bytes, void* stream);
+/* Top-k with per-group caps (a varied practice set: at most c_j problems of group j).  Group masks first: for candidate
+ * c < n (n as for kgat_recommend_topk), bit g of masks[4 c + g / 32] (bit g % 32) is set iff CSR row user_num + cand_items[c]
+ * of A stores a column among group_nodes[group_ptr[g] .. group_ptr[g+1]) -- the membership test of kgat_recommend_filter.
+ * n_groups in [0, 128]; masks uint32 [n_cand_max, 4].  One launch, no host synchronisation. */
+int kgat_recommend_group_masks(const int32_t* row_ptr, const int32_t* col_idx, int64_t n_nodes, int32_t user_num, const int32_t* cand_items,
+                               int64_t n_cand_max, const int32_t* n_cand, const int32_t* group_ptr, const int32_t* group_nodes, int32_t n_groups,
+                               uint32_t* masks, void* stream);
+/* Then rounds r = 0, 1, ... of the exact greedy: for row b, walk its eligible candidates (as for kgat_recommend_topk) in
+ * kgat_recommend_topk's order and accept c when every group g of c has count_g < caps[g] (int32 [n_groups], each >= 0);
+ * accepting adds 1 to count_g for each group of c; stop at k acceptances.  Round r takes, for each
+ * of its n_active rows, the top m (k <= m <= 128) candidates after the row's last entry of round r - 1 that touch no group
+ * already at its cap, and walks them.  A row is finished when it has k entries or the round found fewer than m; the others
+ * go to round r + 1, *n_active_next of them (device int32, written by the call).  Round 0 takes n_active = n_users; call
+ * the next round with the value read back from *n_active_next until it is 0, with the same arguments and workspace
+ * otherwise.  At most n_groups + 1 rounds.  Outputs, complete once no row is active:
+ *   out_items  int64 [n_users, k]  cand_items of the accepted candidates in acceptance order, -1 after out_count[b]
+ *   out_scores fp32  [n_users, k]  their scores (bit-identical to kgat_recommend_topk), -inf after out_count[b]
+ *   out_count  int32 [n_users]     number of accepted candidates
+ * slices in [0, 64] (0 = the rule of kgat_recommend_topk, applied to each round's active rows; the result does not depend
+ * on it).  Two launches per round, no host synchronisation; workspace from kgat_recommend_capped_workspace_bytes with the
+ * same arguments (-1 for invalid ones, or a row too wide for shared memory at m, when the round returns KGAT_ERR_UNSUPPORTED). */
+int64_t kgat_recommend_capped_workspace_bytes(const kgat_tables_t* tables, int64_t n_users, int64_t n_cand_max, int32_t n_groups, int32_t k,
+                                              int32_t m, int32_t slices);
+int kgat_recommend_capped_round(const kgat_tables_t* tables, const int32_t* users, int64_t n_users, const int32_t* cand_items, int64_t n_cand_max,
+                                const int32_t* n_cand, const uint32_t* masks, const int32_t* caps, int32_t n_groups, int32_t k, int32_t m,
+                                const int32_t* exclude_ptr, const int32_t* exclude_items, int32_t slices, int32_t round, int64_t n_active,
+                                int32_t* n_active_next, int64_t* out_items, float* out_scores, int32_t* out_count, void* workspace,
+                                int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* Exact full ranking of held-out targets (the full-ranking metrics: rank, MRR, AUC, any k)      */

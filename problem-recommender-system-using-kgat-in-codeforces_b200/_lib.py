@@ -13,7 +13,7 @@ from pathlib import Path
 
 KGAT_MAX_LAYERS = 8
 KGAT_MAX_TENSORS = 24
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 _PKG_DIR = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ.get("KGAT_B200_LIB", _PKG_DIR / "lib" / "libkgat_b200.so"))
@@ -125,6 +125,10 @@ SIGNATURES: dict[str, tuple] = {
     "kgat_recommend_filter": (_I32, [_P, _P, _I64, _I32, _P, _I64, _P, _P, _I32, _P, _P, _P, _P]),
     "kgat_recommend_workspace_bytes": (_I64, [C.POINTER(TablesT), _I64, _I64, _I32, _I32]),
     "kgat_recommend_topk": (_I32, [C.POINTER(TablesT), _P, _I64, _P, _I64, _P, _I32, _P, _P, _I32, _P, _P, _P, _P, _I64, _P]),
+    "kgat_recommend_group_masks": (_I32, [_P, _P, _I64, _I32, _P, _I64, _P, _P, _P, _I32, _P, _P]),
+    "kgat_recommend_capped_workspace_bytes": (_I64, [C.POINTER(TablesT), _I64, _I64, _I32, _I32, _I32, _I32]),
+    "kgat_recommend_capped_round": (_I32, [C.POINTER(TablesT), _P, _I64, _P, _I64, _P, _P, _P, _I32, _I32, _I32, _P, _P, _I32, _I32, _I64, _P, _P,
+                                           _P, _P, _P, _I64, _P]),
     "kgat_rank_workspace_bytes": (_I64, [C.POINTER(TablesT), _I64, _I64]),
     "kgat_rank_targets": (_I32, [C.POINTER(TablesT), _P, _I64, _P, _I64, _P, _I64, _P, _P, _P, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _I64, _P]),
     "kgat_complete_workspace_bytes": (_I64, [_I32, _I32, _I64, _I64, _I64, _I32, _I32, _I32, _I32]),
@@ -172,7 +176,8 @@ KERNELS_PER_CALL = {
     "kgat_frontier_list": 2, "kgat_frontier_zero_rows": 1, "kgat_frontier_segment": 1, "kgat_biagg_forward_rows": 1, "kgat_biagg_backward_rows": 1, "kgat_biagg_forward": 1, "kgat_biagg_backward": 1,
     "kgat_biagg_reduce_param_grads": 1, "kgat_bpr_forward": 2, "kgat_bpr_backward": 1, "kgat_transr_forward": 2,
     "kgat_transr_backward": 1, "kgat_att_pair_scores": 1, "kgat_mha_forward": 1, "kgat_att_pair_project": 1, "kgat_att_edge_scores_kgat": 1, "kgat_att_edge_scores_dropout": 1, "kgat_att_row_softmax": 1,
-    "kgat_att_edge_weights": 1, "kgat_gather_concat": 1, "kgat_sgemm_nt": 1, "kgat_mask_scores": 1, "kgat_topk_rows": 1, "kgat_explain_paths": 2, "kgat_recommend_filter": 2, "kgat_recommend_topk": 2, "kgat_rank_targets": 3,
+    "kgat_att_edge_weights": 1, "kgat_gather_concat": 1, "kgat_sgemm_nt": 1, "kgat_mask_scores": 1, "kgat_topk_rows": 1, "kgat_explain_paths": 2, "kgat_recommend_filter": 2, "kgat_recommend_topk": 2, "kgat_recommend_group_masks": 1,
+    "kgat_recommend_capped_round": 2, "kgat_rank_targets": 3,
     "kgat_complete_topk": 3, "kgat_complete_rank": 7,
     "kgat_adam_advance": 1, "kgat_adam_set_hyper": 1, "kgat_adam_apply": 1, "kgat_adam_hyper_table": 1, "kgat_adam_lazy_catchup": 1, "kgat_adam_sparse_rows": 1,
     "kgat_adam_lazy_flush": 1, "kgat_fill_f32": 1, "kgat_select_batch_i64": 1, "kgat_sample_cf_batch": 1, "kgat_sample_kg_batch": 1,

@@ -18,7 +18,7 @@ import os
 import torch
 
 from . import _lib, ops
-from .functions import DropoutSpec, last_table_grad, propagate_backward, propagate_forward
+from .functions import DropoutSpec, capture_graph, last_table_grad, propagate_backward, propagate_forward
 from .model import KGAT, KGATMode
 from .optim import FusedAdam
 from .trainer import CF_BATCH, KG_BATCH, EpochData
@@ -307,7 +307,7 @@ class TrainEngine:
                 self.kg_grads[0].zero_()
             g = torch.cuda.CUDAGraph()
             before = _lib.LaunchCounter.count
-            with torch.cuda.graph(g):
+            with capture_graph(g):
                 body(select)
             kernels = _lib.LaunchCounter.count - before  # our kernels recorded in this graph
             _lib.LaunchCounter.count = before

@@ -12,6 +12,8 @@ BPR kernels gather from the four tables directly (K3 of SURVEY.md section 2b).
 
 from __future__ import annotations
 
+import contextlib
+import gc
 from dataclasses import dataclass, field
 
 import torch
@@ -250,6 +252,22 @@ class KGLossFunction(torch.autograd.Function):
 # ----------------------------------------------------------------------------------------------
 # CUDA-graph fast path behind the reference-facing API (model(...), loss.backward(), update_*_weights(), loss.item())
 # ----------------------------------------------------------------------------------------------
+@contextlib.contextmanager
+def capture_graph(graph: torch.cuda.CUDAGraph):
+    """``torch.cuda.graph(graph)`` with Python's cyclic garbage collector paused during the capture.  Captured steps and
+    optimiser plans sit in reference cycles, so an unreachable one is destroyed whenever a collection runs; a collection in the
+    middle of a capture would destroy its CUDAGraph there, with CUDA calls that a capturing stream does not permit, and
+    invalidate the capture.  ``torch.cuda.graph`` collects once before the capture begins."""
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph):
+            yield
+    finally:
+        if enabled:
+            gc.enable()
+
+
 class GraphedStep:
     """One training mode's forward AND backward captured as ONE CUDA graph over static buffers.
 
@@ -317,7 +335,7 @@ class GraphedStep:
         self.ring.zero_()
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
+        with capture_graph(self.graph):
             self.grads = whole(self)
         self._exec = self.graph.raw_cuda_graph_exec()
         self._ids_ptr = self.ids.data_ptr()

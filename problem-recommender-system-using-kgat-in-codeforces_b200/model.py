@@ -666,6 +666,46 @@ class KGAT(nn.Module):
         out_items, scores, count = ops.launch_recommend_topk(tables, users32, cand32, k, ex_ptr, ex_items, n_cand=n_cand)
         return Recommendation(items=out_items, scores=scores, count=count)
 
+    @torch.no_grad()
+    def recommend_capped(self, user_ids, items, k, caps, exclude=None, require=None) -> "Recommendation":
+        """Each user's top-``k`` problems with at most ``cap`` problems of each capped group: a varied practice set, e.g.
+        ``caps=[([t], 3) for t in tags] + [([r], 4) for r in ratings] + [([geometry], 0)]``.
+
+        ``user_ids``, ``items``, ``k``, ``exclude`` and ``require`` mean what they mean for ``recommend``.  ``caps``: a list of at
+        most 128 ``(group, cap)`` pairs, a group a non-empty list of entity ids and a cap an int >= 0.  Problem ``p`` is a member
+        of a group when the current ``attentive_matrix`` stores an entry at ``(user_num + p, user_num + e)`` for some ``e`` of the
+        group -- ``require``'s membership rule.  For every row, the eligible problems (``items``, then ``require``, minus
+        ``exclude[u]``) are walked in ``recommend``'s order, score descending then earlier position in ``items``; ``p`` is
+        accepted when every capped group it is a member of holds fewer than ``cap`` accepted problems so far, and the walk
+        stops at ``k`` acceptances.  A problem in no capped group is always accepted; cap 0 keeps a group out entirely.
+
+        Returns the accepted problems in acceptance order with their fp32 ``PREDICT`` scores, bit-identical to ``recommend``'s,
+        and ``count``; positions from ``count`` on hold -1 / -inf.  With every cap >= ``k`` the result equals ``recommend``'s.
+        The exact answer can lie arbitrarily deep in the ranking, so the GPU works in rounds (at most one per group plus one)
+        and the host reads the number of unfinished rows after each.  ValueError for every argument ``recommend`` rejects and
+        for malformed ``caps``.  Uses the cached propagation after settling deferred KG rows, draws no random numbers, and
+        honours train / eval mode as PREDICT does: call it in ``eval()``."""
+        k = int(k)
+        if not 1 <= k <= 128:
+            raise ValueError(f"k must be in [1, 128], got {k}")
+        dev = self._device()
+        users, cand = self._users_and_items(user_ids, items, exclude)
+        groups, cap_values = ops.cap_groups(caps, self._entity_num)
+        if require is not None:
+            require = ops.require_groups(require, self._entity_num)
+        dup = ops.duplicate_count(cand)
+        users32, cand32 = ops.range_check([("user ids", users, self._user_num), ("item ids", cand, self._entity_num)], dev,
+                                          flags=[("items holds duplicate ids", dup)])
+        tables = self._tables()
+        graph = self._graph()
+        n_cand = None
+        if require is not None:
+            _, cand32, n_cand = ops.launch_recommend_filter(graph, cand32, require, self._user_num)
+        ex_ptr, ex_items = (exclude.ptr_dev.to(dev), exclude.items.to(dev)) if exclude is not None else (None, None)
+        out_items, scores, count, _ = ops.launch_recommend_capped(tables, graph, users32, cand32, k, groups, cap_values, self._user_num, ex_ptr,
+                                                                  ex_items, n_cand=n_cand)
+        return Recommendation(items=out_items, scores=scores, count=count)
+
     def _users_and_items(self, user_ids, items, exclude):
         """``user_ids`` / ``items`` of ``recommend`` and ``rank`` as int64 on the device (ranges are checked by the caller's
         read-back); ValueError for a malformed argument or an ``exclude`` over another number of users."""

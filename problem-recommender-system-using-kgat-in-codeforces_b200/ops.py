@@ -9,6 +9,7 @@ op when the library or a GPU is missing -- the call raises.
 from __future__ import annotations
 
 import ctypes as C
+import operator
 
 import torch
 
@@ -776,19 +777,24 @@ def recommend_filter(graph, items: torch.Tensor, groups, user_num: int):
     return launch_recommend_filter(graph, items32, groups, user_num)
 
 
+def _group_nodes(groups, user_num: int, dev):
+    """Groups of entity ids as a CSR over CKG node ids: (group_ptr int32 [G + 1], group_nodes int32), on ``dev``."""
+    gptr = torch.tensor([0] + [len(g) for g in groups], dtype=i64).cumsum(0).to(dtype=i32, device=dev)
+    gnodes = torch.tensor([e for g in groups for e in g], dtype=i32).add_(user_num).to(dev)
+    return gptr, gnodes
+
+
 def launch_recommend_filter(graph, items32: torch.Tensor, groups, user_num: int):
     """``recommend_filter`` for int32 ``items32`` and ``groups`` already known to lie in range (no checks, no synchronisation)."""
     lib = _lib.load()
     dev = graph.col_idx.device
-    flat = [e for g in groups for e in g]
-    gptr = torch.tensor([0] + [len(g) for g in groups], dtype=i64).cumsum(0).to(dtype=i32, device=dev)
-    gnodes = torch.tensor(flat, dtype=i32).add_(user_num).to(dev)
+    gptr, gnodes = _group_nodes(groups, user_num, dev)
     n = items32.numel()
     positions = torch.empty(n, dtype=i32, device=dev)
     cand = torch.zeros(n, dtype=i32, device=dev)  # entries from n_cand on stay 0, a valid row for recommend_topk_fused's range check
     n_cand = torch.empty(1, dtype=i32, device=dev)
     check(lib.kgat_recommend_filter(_ptr(graph.row_ptr, i32), _ptr(graph.col_idx, i32), graph.n, user_num, _ptr(items32, i32, "items") if n else None,
-                                    n, gptr.data_ptr(), gnodes.data_ptr() if flat else None, len(groups), positions.data_ptr() if n else None,
+                                    n, gptr.data_ptr(), gnodes.data_ptr() if gnodes.numel() else None, len(groups), positions.data_ptr() if n else None,
                                     cand.data_ptr() if n else None, n_cand.data_ptr(), _stream()), "recommend_filter")
     return positions, cand, n_cand
 
@@ -845,6 +851,115 @@ def launch_recommend_topk(tables, users32: torch.Tensor, cand32: torch.Tensor, k
         None if exclude_ptr is None else _ptr(exclude_ptr, i32, "exclude_ptr"), None if exclude_items is None else _ptr(exclude_items, i32, "exclude_items"),
         s, out_items.data_ptr(), out_scores.data_ptr(), out_count.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "recommend_topk")
     return out_items, out_scores, out_count
+
+
+def cap_groups(caps, n_ent: int):
+    """``caps`` of ``recommend_capped``, a list of ``(group, cap)`` pairs, as (groups: lists of ints, caps: ints); ValueError for
+    more than 128 pairs, an empty group, an entity id outside ``[0, n_ent)``, or a cap that is not an integer >= 0."""
+    try:
+        pairs = [(list(g), c) for g, c in caps]
+    except (TypeError, ValueError):
+        raise ValueError("caps must be a list of (group, cap) pairs") from None
+    if len(pairs) > 128:
+        raise ValueError(f"at most 128 capped groups, got {len(pairs)}")
+    groups, values = [], []
+    for g, c in pairs:
+        if isinstance(c, bool) or (isinstance(c, torch.Tensor) and c.dtype == torch.bool):
+            raise ValueError(f"a cap must be an integer >= 0, got {c!r}")
+        try:
+            c = operator.index(c)
+        except TypeError:
+            raise ValueError(f"a cap must be an integer >= 0, got {c!r}") from None
+        if c < 0:
+            raise ValueError(f"a cap must be an integer >= 0, got {c}")
+        if len(g) == 0:
+            raise ValueError("every group of `caps` must hold at least one entity id")
+        g = [int(e) for e in g]
+        if any(not 0 <= e < n_ent for e in g):
+            raise ValueError(f"entity ids of `caps` must lie in [0, {n_ent})")
+        groups.append(g)
+        values.append(c)
+    return groups, values
+
+
+def recommend_capped(tables, graph, users: torch.Tensor, cand_items: torch.Tensor, k: int, caps, user_num: int, exclude_ptr=None,
+                     exclude_items=None, m=None, slices=None):
+    """Top-``k`` of ``cand_items`` for every row of ``users`` with at most ``cap`` problems of each capped group, in one call
+    (``kgat_recommend_group_masks`` + ``kgat_recommend_capped_round``).  ``tables``, ``users``, ``cand_items``, ``exclude_*`` and
+    ``slices`` as for ``recommend_topk_fused``; ``graph``: the ``AttentiveGraph`` whose rows give group membership (problem ``p``
+    is in a group when row ``user_num + p`` stores ``user_num + e`` for some ``e`` of it); ``caps``: list of ``(group, cap)``
+    pairs (see ``cap_groups``); ``m`` (``k`` .. 128, None = ``max(k, 64)``): candidates per row and round.
+    Each row walks its candidates in ``recommend_topk_fused``'s order and accepts one when all its groups are below their caps,
+    until ``k`` are accepted.  Returns ``(items int64 [U, k], scores fp32 [U, k], count int32 [U], rounds)``, padded with
+    -1 / -inf after ``count``; neither ``m`` nor ``slices`` changes the result."""
+    k = int(k)
+    if not 1 <= k <= 128:
+        raise ValueError(f"k must be in [1, 128], got {k}")
+    if m is not None and not k <= int(m) <= 128:
+        raise ValueError(f"m must be in [k, 128] = [{k}, 128], got {m}")
+    if slices is not None and not 1 <= int(slices) <= 64:
+        raise ValueError(f"slices must be in [1, 64], got {slices}")
+    if (exclude_ptr is None) != (exclude_items is None):
+        raise ValueError("exclude_ptr and exclude_items go together")
+    user_num = int(user_num)
+    if not 0 <= user_num < graph.n:
+        raise ValueError(f"user_num {user_num} outside [0, {graph.n})")
+    groups, values = cap_groups(caps, graph.n - user_num)
+    dev = tables[0].device
+    rows = tables[0].shape[0]
+    users = _ids64(users, "users", dev)
+    cand_items = _ids64(cand_items, "cand_items", dev)
+    checks = [("user ids", users, rows), ("candidate ids", cand_items, min(rows, graph.n - user_num))]
+    if exclude_ptr is not None:
+        if exclude_ptr.dim() != 1 or exclude_ptr.numel() < 2:
+            raise ValueError("exclude_ptr must be 1-D with one entry per user row plus one")
+        checks.append(("user ids (rows of exclude_ptr)", users, exclude_ptr.numel() - 1))
+    users32, cand32 = range_check(checks, dev)[:2]
+    return launch_recommend_capped(tables, graph, users32, cand32, k, groups, values, user_num, exclude_ptr, exclude_items, m, slices)
+
+
+def launch_recommend_capped(tables, graph, users32: torch.Tensor, cand32: torch.Tensor, k: int, groups, caps, user_num: int, exclude_ptr=None,
+                            exclude_items=None, m=None, slices=None, n_cand=None, active_rows=None):
+    """``recommend_capped`` for int32 ids and arguments already known to be valid (``groups`` / ``caps`` from ``cap_groups``);
+    ``n_cand`` (device int32 [1], e.g. from ``recommend_filter``): only the first ``n_cand`` candidates count; ``active_rows``: a
+    list that receives the number of rows of each round.  No checks; one host synchronisation per round, to read the number
+    of rows still active."""
+    lib = _lib.load()
+    dev = tables[0].device
+    t = _tables(tables)
+    U, n, G = users32.numel(), cand32.numel(), len(groups)
+    m = max(k, 64) if m is None else int(m)
+    out_items = torch.empty(U, k, dtype=i64, device=dev)
+    out_scores = torch.empty(U, k, dtype=f32, device=dev)
+    out_count = torch.empty(U, dtype=i32, device=dev)
+    if U == 0:
+        return out_items, out_scores, out_count, 0
+    s = 0 if slices is None else int(slices)
+    ws_bytes = int(lib.kgat_recommend_capped_workspace_bytes(C.byref(t), U, n, G, k, m, s))
+    if ws_bytes < 0:
+        raise KgatLibraryError(f"recommend_capped: tables of width {sum(x.shape[1] for x in tables)} rejected (not multiples of 4, or too wide for shared memory at m = {m})")
+    ws = torch.empty(max(ws_bytes, 1), dtype=u8, device=dev)
+    gptr, gnodes = _group_nodes(groups, user_num, dev)
+    caps_dev = torch.tensor(caps, dtype=i32).to(dev)
+    masks = torch.empty(n, 4, dtype=i32, device=dev)
+    n_cand_p = None if n_cand is None else _ptr(n_cand, i32, "n_cand")
+    check(lib.kgat_recommend_group_masks(_ptr(graph.row_ptr, i32), _ptr(graph.col_idx, i32), graph.n, user_num, _ptr(cand32, i32, "cand_items") if n else None,
+                                         n, n_cand_p, gptr.data_ptr(), gnodes.data_ptr() if G else None, G, masks.data_ptr() if n else None, _stream()),
+          "recommend_group_masks")
+    ex_p = None if exclude_ptr is None else _ptr(exclude_ptr, i32, "exclude_ptr")
+    ex_i = None if exclude_items is None else _ptr(exclude_items, i32, "exclude_items")
+    n_next = torch.zeros(1, dtype=i32, device=dev)
+    n_active, rounds = U, 0
+    while n_active:
+        if active_rows is not None:
+            active_rows.append(n_active)
+        check(lib.kgat_recommend_capped_round(
+            C.byref(t), _ptr(users32, i32, "users"), U, _ptr(cand32, i32, "cand_items") if n else None, n, n_cand_p, masks.data_ptr() if n else None,
+            caps_dev.data_ptr() if G else None, G, k, m, ex_p, ex_i, s, rounds, n_active, n_next.data_ptr(), out_items.data_ptr(),
+            out_scores.data_ptr(), out_count.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "recommend_capped_round")
+        rounds += 1
+        n_active = int(n_next.item())
+    return out_items, out_scores, out_count, rounds
 
 
 def duplicate_count(ids: torch.Tensor) -> torch.Tensor:

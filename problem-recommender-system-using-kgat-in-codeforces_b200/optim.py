@@ -12,6 +12,7 @@ from __future__ import annotations
 import torch
 
 from . import ops
+from .functions import capture_graph
 
 
 class DeferredRows:
@@ -110,7 +111,7 @@ class FusedAdam(torch.optim.Optimizer):
             params, grads = [p.data for p in ps], [p.grad for p in ps]
             ms, vs = [self.state[p]["exp_avg"] for p in ps], [self.state[p]["exp_avg_sq"] for p in ps]
             torch.cuda.synchronize()
-            with torch.cuda.graph(plan["graph"]):
+            with capture_graph(plan["graph"]):
                 ops.adam_advance(plan["step_dev"], group["lr"], beta1, beta2, group["eps"], plan["hyper"])
                 ops.adam_apply(params, grads, ms, vs, plan["hyper"])
             self._plans[key] = plan
@@ -181,12 +182,12 @@ class FusedAdam(torch.optim.Optimizer):
                 # the step's own advance + (claimed rows, small dense tensors, window slice) in one launch; the captured step_dev /
                 # row_step contents are restored below (the capture itself does not run anything)
                 h, pt, nt = rolling["ids"]
-                with torch.cuda.graph(plan["graph"]):
+                with capture_graph(plan["graph"]):
                     ops.adam_advance(d.step_dev, group["lr"], beta1, beta2, group["eps"], d.hyper)
                     ops.adam_rolling_apply(h, pt, nt, rolling["row_slot"], grads[0], params[0], ms[0], vs[0], d.row_step, d.window,
                                            params[1:], list(grads)[1:], ms[1:], vs[1:], d.step_dev, d.s0, d.table, d.hyper)
             else:
-                with torch.cuda.graph(plan["graph"]):
+                with capture_graph(plan["graph"]):
                     ops.adam_advance(plan["step_dev"], group["lr"], beta1, beta2, group["eps"], plan["hyper"])
                     ops.adam_apply(params, list(grads), ms, vs, plan["hyper"], row_slot0=row_slot0)
             plan["exec"] = plan["graph"].raw_cuda_graph_exec()

@@ -36,7 +36,7 @@ import torch.distributed as dist
 from . import _lib, ops
 from .engine import TrainEngine
 from .frontier import Frontier
-from .functions import DropoutSpec, _buf, last_table_grad
+from .functions import DropoutSpec, _buf, capture_graph, last_table_grad
 from .model import KGATMode
 from .peer import PeerArena
 
@@ -341,7 +341,7 @@ class RangeShardedEngine:
             self.arena.signal_wait(4)
             g = torch.cuda.CUDAGraph()
             before = _lib.LaunchCounter.count
-            with torch.cuda.graph(g):
+            with capture_graph(g):
                 self._cf_graphed_step()
             self._cf_kernels = _lib.LaunchCounter.count - before
             _lib.LaunchCounter.count = before

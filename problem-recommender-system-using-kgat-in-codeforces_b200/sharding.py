@@ -528,10 +528,11 @@ class ShardedEngine:
             if self.part.world > 1:
                 dist.barrier()
             from . import _lib
+            from .functions import capture_graph
 
             g = torch.cuda.CUDAGraph()
             before = _lib.LaunchCounter.count
-            with torch.cuda.graph(g):
+            with capture_graph(g):
                 self._cf_graphed_step()
             self._cf_kernels = _lib.LaunchCounter.count - before
             _lib.LaunchCounter.count = before
