@@ -334,11 +334,8 @@ int launch_pairs(const float* emb, const float* W, const int32_t* pt, const int3
                  float* score_out, cudaStream_t stream) {
     constexpr int D = DM * 32;
     const size_t smem = sizeof(float) * 2 * D * D;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(pair_scores_kernel<DM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(pair_scores_kernel<DM>, (int)smem, configured); rc != KGAT_OK) return rc;
     int64_t blocks = (n_pairs + 3) / 4;
     const int64_t cap = (int64_t)sm_count() * (DM <= 2 ? 4 : 1);
     if (blocks > cap) blocks = cap;
@@ -351,11 +348,8 @@ int launch_edges(const float* pair_v, const int32_t* poe, int64_t n_edges, const
                  uint64_t offset, const uint64_t* seed_dev, float* score_out, cudaStream_t stream) {
     constexpr int D = DM * 32;
     const size_t smem = sizeof(float) * D * D;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(edge_scores_dropout_kernel<DM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(edge_scores_dropout_kernel<DM>, (int)smem, configured); rc != KGAT_OK) return rc;
     int64_t blocks = (n_edges + 3) / 4;
     const int64_t cap = (int64_t)sm_count() * (DM <= 2 ? 8 : 2);
     if (blocks > cap) blocks = cap;
@@ -369,11 +363,8 @@ int launch_mha(const float* x, int64_t n, const Mha& P, float p, const uint8_t* 
                cudaStream_t stream) {
     constexpr int D = DM * 32;
     const size_t smem = sizeof(float) * 2 * D * D;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(mha_forward_kernel<DM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(mha_forward_kernel<DM>, (int)smem, configured); rc != KGAT_OK) return rc;
     int64_t blocks = (n + 3) / 4;
     const int64_t cap = (int64_t)sm_count() * (DM <= 2 ? 4 : 1);
     if (blocks > cap) blocks = cap;

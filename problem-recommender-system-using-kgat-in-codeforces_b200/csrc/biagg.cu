@@ -392,11 +392,8 @@ int launch_fwd(const float* E, const float* S, int64_t n, const float* W1, const
                float p, uint64_t seed, uint64_t offset, const uint64_t* seed_dev, const uint32_t* keep_bits, float* out, int64_t ld_out,
                float* inv_norm, uint8_t* flags, cudaStream_t stream) {
     using C = Cfg<DIN, DOUT>;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(biagg_fwd_kernel<DIN, DOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::fwd_smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(biagg_fwd_kernel<DIN, DOUT>, (int)C::fwd_smem, configured); rc != KGAT_OK) return rc;
     const int grid = grid_for(n, C::TM, C::fwd_smem);
     biagg_fwd_kernel<DIN, DOUT><<<grid, C::NT, C::fwd_smem, stream>>>(E, S, n, W1, b1, W2, b2, p, seed, offset, seed_dev, keep_bits,
                                                                      out, ld_out, inv_norm, flags);
@@ -408,11 +405,8 @@ int launch_bwd(const float* g_out, int64_t ld_gout, const float* out, int64_t ld
                const float* E, const float* S, int64_t n, const float* W1, const float* W2, float p, float* g_S, float* g_E,
                float* partials, int n_ctas, cudaStream_t stream) {
     using C = Cfg<DIN, DOUT>;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(biagg_bwd_kernel<DIN, DOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::bwd_smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(biagg_bwd_kernel<DIN, DOUT>, (int)C::bwd_smem, configured); rc != KGAT_OK) return rc;
     biagg_bwd_kernel<DIN, DOUT><<<n_ctas, C::NT, C::bwd_smem, stream>>>(g_out, ld_gout, out, ld_out, inv_norm, flags, E, S, n, W1, W2,
                                                                        p, g_S, g_E, partials);
     return check_launch();

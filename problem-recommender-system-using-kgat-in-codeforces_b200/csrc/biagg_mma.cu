@@ -537,11 +537,8 @@ int launch_fwd(const float* E, const float* S, int64_t n, const float* W1, const
                float* inv_norm, uint8_t* flags, float* const* peer_out, int n_peers, const int32_t* row_ids, const int32_t* n_dev,
                cudaStream_t stream) {
     using C = FwdCfg<DIN, DOUT>;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(biagg_fwd_mma_kernel<DIN, DOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(biagg_fwd_mma_kernel<DIN, DOUT>, (int)C::smem, configured); rc != KGAT_OK) return rc;
     biagg_fwd_mma_kernel<DIN, DOUT><<<grid_for(n, C::TM, C::smem), C::NT, C::smem, stream>>>(E, S, n, W1, b1, W2, b2, p, seed, offset, seed_dev,
                                                                                          keep_bits, out, ld_out, inv_norm, flags, peer_out,
                                                                                          n_peers, row_ids, n_dev);
@@ -554,11 +551,8 @@ int launch_bwd(const float* g_out, int64_t ld_gout, const float* out, int64_t ld
                float* partials, int n_ctas, float* const* peer_gS, int n_peers, const int32_t* row_ids, const int32_t* n_dev,
                cudaStream_t stream) {
     using C = BwdCfg<DIN, DOUT>;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(biagg_bwd_mma_kernel<DIN, DOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(biagg_bwd_mma_kernel<DIN, DOUT>, (int)C::smem, configured); rc != KGAT_OK) return rc;
     biagg_bwd_mma_kernel<DIN, DOUT><<<n_ctas, C::NT, C::smem, stream>>>(g_out, ld_gout, out, ld_out, inv_norm, flags, E, S, n, W1, W2, p, g_S,
                                                                     g_E, partials, peer_gS, n_peers, row_ids, n_dev);
     return check_launch();

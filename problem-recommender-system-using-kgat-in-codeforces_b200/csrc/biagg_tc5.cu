@@ -331,11 +331,8 @@ int launch_fwd(const float* E, const float* S, int64_t n, const float* W1, const
                float* inv_norm, uint8_t* flags, float* const* peer_out, int n_peers, const int32_t* row_ids, const int32_t* n_dev,
                cudaStream_t stream) {
     using C = Cfg<DIN, DOUT>;
-    static bool configured = false;
-    if (!configured) {
-        KGAT_CUDA_TRY(cudaFuncSetAttribute(biagg_fwd_tc5_kernel<DIN, DOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
-        configured = true;
-    }
+    static uint64_t configured = 0;
+    if (const int rc = raise_smem_limit(biagg_fwd_tc5_kernel<DIN, DOUT>, (int)C::smem, configured); rc != KGAT_OK) return rc;
     const int64_t tiles = (n + C::TM - 1) / C::TM;
     const int grid = (int)(tiles < sm_count() ? tiles : sm_count());
     biagg_fwd_tc5_kernel<DIN, DOUT><<<grid, C::NT, C::smem, stream>>>(E, S, n, W1, b1, W2, b2, p, seed, offset, seed_dev, keep_bits, out,

@@ -46,6 +46,21 @@ inline int sm_count() {
         }                                    \
     } while (0)
 
+// Raise a kernel's dynamic shared-memory limit to `bytes` on the current device, once per device: the attribute belongs to
+// each device's copy of the function, so a process that launches the kernel on cuda:0 and then on cuda:1 sets it twice.
+// `configured` is the launcher's static record, one bit per device.
+template <class Kernel>
+inline int raise_smem_limit(Kernel* kernel, int bytes, uint64_t& configured) {
+    int dev = 0;
+    KGAT_CUDA_TRY(cudaGetDevice(&dev));
+    const uint64_t bit = 1ull << (dev & 63);
+    if (!(configured & bit)) {
+        KGAT_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        configured |= bit;
+    }
+    return KGAT_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // device helpers
 // ------------------------------------------------------------------------------------------

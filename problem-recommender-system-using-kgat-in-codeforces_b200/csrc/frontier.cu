@@ -286,11 +286,8 @@ int kgat_frontier_expand(const int32_t* tasks, int64_t n_heavy_tasks, const int3
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n_words = (n_nodes + 31) / 32;
     if (!plain && n_words * 4 <= 200 * 1024) {
-        static bool configured = false;
-        if (!configured) {
-            KGAT_CUDA_TRY(cudaFuncSetAttribute(frontier_expand_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            configured = true;
-        }
+        static uint64_t configured = 0;
+        if (const int rc = raise_smem_limit(frontier_expand_smem_kernel, 200 * 1024, configured); rc != KGAT_OK) return rc;
         int64_t big = (max_rows + n_heavy_tasks + 31) / 32;
         if (big > sm_count()) big = sm_count();
         frontier_expand_smem_kernel<<<(unsigned)big, 1024, (size_t)n_words * 4, st>>>(t4, (int)n_heavy_tasks, light_rank, col_idx, rows, count_dev,
