@@ -36,6 +36,7 @@ class SpmmPlan:
     n_tasks: int
     n_heavy: int
     n_partials: int  # = number of heavy-chunk tasks; they come first in `tasks`
+    n_rows: int  # rows of the matrix: an output (and an addend) needs at least this many
     light_rank: torch.Tensor | None = None  # int32 [n_rows]: a light row's task is n_partials + light_rank[row]; -1 = heavy row
 
 
@@ -85,6 +86,7 @@ def make_plan(row_ptr: torch.Tensor, chunk: int = DEFAULT_CHUNK) -> SpmmPlan:
         n_tasks=int(tasks.shape[0]),
         n_heavy=int(heavy.shape[0]),
         n_partials=n_partials,
+        n_rows=int(rp.shape[0] - 1),
         light_rank=torch.from_numpy(light_rank).to(dev).contiguous(),
     )
 

@@ -213,8 +213,12 @@ def spmm(plan, col_idx, vals, x: torch.Tensor, out: torch.Tensor, addend: torch.
     ``frontier.Frontier`` level (only the rows in ``row_mask`` are computed; edges / addend rows outside ``edge_mask`` are
     dropped).  With the level's row list (``rows``, ``n_rows_dev``; needs ``row_mask`` too) or with an ``edge_mask`` alone the
     persistent row-list kernel runs; a ``row_mask`` without a list uses the grid-per-task kernel."""
-    lib = _lib.load()
     d = x.shape[1]
+    # the kernels write d floats at row * ld of every plan row: a narrower or shorter output would be written out of bounds
+    for name, t in (("out", out), ("addend", addend)):
+        if t is not None and (t.dim() != 2 or t.shape[1] != d or t.shape[0] < plan.n_rows):
+            raise KgatLibraryError(f"spmm: {name} of shape {tuple(t.shape)} does not cover {plan.n_rows} rows of width {d}")
+    lib = _lib.load()
     if plan.n_heavy > 0:
         need = plan.n_partials * d
         if partials is None or partials.numel() < need:
@@ -259,8 +263,11 @@ def spmm_scatter_rows(plan, col_idx, vals, g: torch.Tensor, out: torch.Tensor, r
                       tag: str = ""):
     """out[c] += A[r, c] * g[r] over the listed rows r (and out[r] += addend[r]); ``plan`` / ``col_idx`` / ``vals`` of A itself.
     The destination rows of ``out`` must have been zeroed (frontier_zero_rows)."""
-    lib = _lib.load()
     d = g.shape[1]
+    for name, t in (("out", out), ("addend", addend)):
+        if t is not None and (t.dim() != 2 or t.shape[1] != d):
+            raise KgatLibraryError(f"spmm_scatter_rows: {name} of shape {tuple(t.shape)} does not have the width {d} of g")
+    lib = _lib.load()
     check(
         lib.kgat_spmm_scatter_rows(
             _ptr(plan.tasks, i32), plan.n_partials, _ptr(plan.light_rank, i32), _ptr(rows, i32), _ptr(n_rows_dev, i32), int(max_rows),
